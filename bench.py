@@ -3,6 +3,7 @@
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
                     [--workload mpc02|mpc02pct5|mpc02pim|socmpc|lp25fv47] [--batch B] [--scaling strong|weak]
+                    [--dump-outputs DIR]
 
 A "step" is one pass of the hot path over one batch: updateData (per-instance h, b) + solve for
 every instance of the batch.  Workload at N=1: BASELINE.json configs[2] - the reference's MPC data
@@ -16,6 +17,9 @@ JSON line (rank 0): value = whole-job solves/s with inputs resident in HBM (devi
 ranks); e2e = the same through the C ABI with HOST buffers (H2D of h,b and D2H of x + exit flags in
 the timed region); roofline = the dominant kernel (eicos_solve_kkt: triangular solves + refinement
 residual) against the measured HBM peak; cpu_baseline = the CPU oracle on this box's host cores.
+--dump-outputs DIR writes what the last timed device-resident step returned (rank 0's instances) as
+DIR/<name>.npy; the inputs are seeded, so two builds run with the same arguments can be compared
+output for output.
 `--impl reference` times the reference path on the host cores: the reference itself needs Eigen,
 which is absent (oracle/Makefile), so it is the oracle port, one solver per core, updateData +
 solve per instance exactly as BASELINE.md section 3 prescribes.
@@ -50,7 +54,31 @@ def parse_args():
                     help="end-to-end arm: handles (one stream and one host thread each) on the device behind eicos_multi_solve; "
                          "copies of one slice overlap the kernels of the others (1 = eicos_batch_solve on the device arm's handle; "
                          "0 = choose: one handle per 16384 instances of this GPU's share, at most 4)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the outputs of the last timed step as DIR/<name>.npy (float64, at most 64 MB in all)")
+    args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of --impl ours")
+    return args
+
+
+DUMP_BYTES = 64_000_000
+
+
+def dump_outputs(out_dir, x, exits, iters):
+    """What the caller of the device-resident path receives: exit.npy and iter.npy of every instance, and x.npy, the
+    solutions of every instance or, where they would not fit DUMP_BYTES, of a fixed seeded sample of the instances
+    (x_instances.npy lists them, in order)."""
+    import torch
+    batch, n = x.shape
+    rows = min(batch, (DUMP_BYTES - 4 * 128 - 16 * batch) // (8 * (n + 1)))  # 128: an .npy header
+    idx = np.arange(batch) if rows == batch else np.sort(np.random.default_rng(0).choice(batch, rows, replace=False))
+    xs = torch.index_select(x, 0, torch.from_numpy(idx).to(x.device)).cpu().numpy()
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in (("x", xs), ("x_instances", idx), ("exit", exits), ("iter", iters)):
+        np.save(os.path.join(out_dir, name + ".npy"), np.ascontiguousarray(a, dtype=np.float64))
 
 
 def make_problem(workload):
@@ -310,6 +338,8 @@ def main():
     value = total_batch * args.steps / (ms * 1e-3)
     exits = exit_d.cpu().numpy()
     iters = iter_d.cpu().numpy()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, x_d, exits, iters)
 
     # ---- end to end through the C ABI with host buffers
     e2e = None

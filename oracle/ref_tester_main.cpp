@@ -1,17 +1,16 @@
-// Runs the reference's OWN test fixtures - test/**/*.h of EmbersArc/EiCOS, compiled unchanged from
-// where they lie under /root/reference, together with the reference's own test/ecos.h shim and
-// test/minunit.h - against THIS repo's drop-in: `#include "eicos.hpp"` in test/ecos.h resolves to
-// include/eicos.hpp (the C++ facade over the C ABI), so every ECOS_setup / ECOS_solve /
-// ECOS_updateData / ECOS_cleanup of the fixtures runs on the engine.  This file is the only part
-// that is ours: the reference's tester main (test/ecostester.cpp) cannot be compiled because it
-// includes MPC/MPC01.h, which is missing from the checkout (SURVEY.md F3), and its mu_assert aborts
-// the process on the first failure - so this main runs ONE named test per process.  The 18 tests
-// are the ones test/ecostester.cpp runs, minus MPC01 (infeasible2.h is dead code in the reference:
-// it is not included by the tester and does not compile against test/ecos.h).
-// TEST INFRASTRUCTURE: built by oracle/Makefile into oracle/_ref/ (never shipped, never loaded by the
-// product).  No reference source is copied into the repository.
+// Runs the tests of the reference's tester (test/ecostester.cpp of EmbersArc/EiCOS) on the engine:
+// fixture headers in the reference's test format (test/**/*.h: data arrays plus a test_<name>()
+// that calls ECOS_setup / ECOS_solve / ECOS_updateData / ECOS_cleanup and asserts the exit flag),
+// found on the include path under the reference's file names.  tests/test_reference_tester.py
+// writes them from the data and expected exit flags stored in tests/golden/fixtures and compiles
+// this file against the ECOS-name shim of tests/cpp/shim.  The 18 tests are the ones
+// test/ecostester.cpp runs, minus MPC01, whose data the reference does not contain (SURVEY.md F3)
+// (infeasible2.h is dead code in the reference: the tester does not include it).  A failed
+// mu_assert ends the process, so this main runs ONE named test per process.
+// TEST INFRASTRUCTURE: never shipped, never loaded by the product.
 #include <cstdio>
 #include <cstring>
+#include <exception>
 
 #include "minunit.h"
 #include "ecos.h"
@@ -34,8 +33,6 @@
 #include "LPnetlib/lp_beaconfd.h"
 #include "LPnetlib/lp_blend.h"
 #include "LPnetlib/lp_bnl1.h"
-
-int tests_run = 0;
 
 namespace
 {
@@ -67,7 +64,7 @@ int main(int argc, char **argv)
         {
             try
             {
-                char *msg = mu_run_test(e.fn); // mu_assert aborts the process when the expectation fails
+                char *msg = e.fn(); // mu_assert ends the process when the expectation fails
                 if (msg)
                 {
                     printf("FAIL %s: %s\n", e.name, msg);
