@@ -190,7 +190,6 @@ void Engine::build_layout(const Symbolic &S, bool acc_rows)
     L.lam = take(S.mt);
     L.wb = take(S.N);
     L.bs = take(S.mt);
-    L.blam = take(S.mt);
     L.r = take(S.N);
     L.lpv = take(S.l);
     L.lpw = take(S.l);
@@ -791,7 +790,7 @@ void Engine::solve(int batch, const double *d_c, const double *d_h, const double
                     // sides (contiguous), scalars
                     // (per-instance matrices: also the equilibrated G / A values and the equilibration vectors)
                     const int rr[14] = {L_.chb, P_.N,
-                                        L_.w, (L_.blam + P_.mt) - L_.w,
+                                        L_.w, (L_.bs + P_.mt) - L_.w,
                                         L_.r, P_.N,
                                         L_.lpv, (L_.V + P_.nnzV) - L_.lpv,
                                         L_.rhs1, 2 * P_.N,

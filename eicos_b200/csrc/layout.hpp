@@ -70,7 +70,7 @@ struct Layout
     int chb;                        // [c | b | h] equilibrated problem vectors, KKT-shaped (N rows)
     int w;                          // current iterate [x | y | z] (N rows)
     int s, lam;                     // slacks, scaled variable (mt rows each)
-    int wb, bs, blam;               // best iterate (w_best)
+    int wb, bs;                     // best iterate (w_best; lambda is not kept: an instance that restores it stops)
     int r;                          // residuals [rx | ry | rz] (N rows)
     int lpv, lpw;                   // LP cone scalings (l rows each)
     int cpar, cq;                   // SOC scalings: CP_COUNT rows per cone, q vectors

@@ -99,6 +99,27 @@ EI_DEV vd vfnma(vd v, double a, vd b)
     VFOR v.v[c_] = fma(-a, b.v[c_], v.v[c_]);
     return v;
 }
+// a * b + c and a * b with one rounding each.  A value recomputed in registers that used to be stored and read
+// back has to round like the stored one, whatever else now uses its parts: these spell out which products the
+// compilers fused where the value was stored (a product whose only use is one add).
+EI_DEV vd vfma(vd a, vd b, vd c)
+{
+    VFOR c.v[c_] = fma(a.v[c_], b.v[c_], c.v[c_]);
+    return c;
+}
+EI_DEV vd vmul_rn(vd a, vd b)
+{
+#ifdef EICOS_EMU
+    VFOR
+    {
+        a.v[c_] *= b.v[c_];
+        asm("" : "+x"(a.v[c_])); // g++: the product is opaque to -ffp-contract
+    }
+#else
+    VFOR a.v[c_] = __dmul_rn(a.v[c_], b.v[c_]);
+#endif
+    return a;
+}
 EI_DEV vd vsqrt(vd a) { VFOR a.v[c_] = sqrt(a.v[c_]); return a; }
 EI_DEV vd vabs(vd a) { VFOR a.v[c_] = fabs(a.v[c_]); return a; }
 EI_DEV bool ei_isnan(double v) { return v != v; }
@@ -1808,6 +1829,12 @@ EI_DEV void tile_resid(const Team &tm, const KArgs &a, int tile)
             ROWD(T, L.sc + S_RED + k) = tot[k];
 }
 
+// lambda = W z of the LP rows.  Without second-order cones it is never stored: its readers take z and recompute
+// lpw * z, rounded alone like the head's product.  With cones the head's cone_scale() writes the rows, and keeps
+// their old values for an instance whose cone scaling failed, so they are read.
+EI_DEV int lp_lambda_row(const DevPattern &P, const Layout &L) { return P.nc == 0 ? L.w + P.n + P.p : L.lam; }
+EI_DEV vd lp_lambda(const DevPattern &P, vd lpw, vd row) { return P.nc == 0 ? vmul_rn(lpw, row) : row; }
+
 // ------------------------------------------------------------------ head of an iteration
 // computeResiduals + updateStatistics + safeguards / exit tests + best-iterate bookkeeping
 // (src/eicos.cpp:997-1158), then for the instances that keep iterating: updateScalings,
@@ -1965,17 +1992,16 @@ EI_DEV void tile_head(const Team &tm, const KArgs &a, int tile)
             ROWC(I, J_STATUS, c_) = codev[c_];
         }
 
-    // ---- vector part of `w = w_best` / `w_best = w`, and backscale (:1271-1277) for finished instances
+    // ---- vector part of `w = w_best` / `w_best = w`, and backscale (:1271-1277) for finished instances.
+    //      lambda is not part of the best iterate here: an instance that restores it always stops, and the lambda
+    //      of a stopped instance is read by nothing.
     if (!tm.any(restore || fin) && tm.all(save || !act))
     { // common case: every active instance improves its best iterate and nobody stops -> plain copies
         // (inactive lanes of w_best are never read again)
         const int ins[1] = {L.w};
         ew_rows<1, 8>(tm, T, P.N, ins, [&](int q, const vd *x) { ROWD(T, L.wb + q) = x[0]; });
-        const int inz[2] = {L.s, L.lam};
-        ew_rows<2, 6>(tm, T, P.mt, inz, [&](int e, const vd *x) {
-            ROWD(T, L.bs + e) = x[0];
-            ROWD(T, L.blam + e) = x[1];
-        });
+        const int inz[1] = {L.s};
+        ew_rows<1, 8>(tm, T, P.mt, inz, [&](int e, const vd *x) { ROWD(T, L.bs + e) = x[0]; });
     }
     else if (tm.any(restore || save || fin))
     {
@@ -1996,17 +2022,15 @@ EI_DEV void tile_head(const Team &tm, const KArgs &a, int tile)
             });
         }
         {
-            const int ins[4] = {L.s, L.lam, L.bs, L.blam};
-            ew_rows<4, 3>(tm, T, P.mt, ins, [&](int e, const vd *x) {
-                vd sv = vsel(restore, x[2], x[0]), lv = vsel(restore, x[3], x[1]);
-                ROWD(T, L.bs + e) = vsel(save, sv, x[2]);
-                ROWD(T, L.blam + e) = vsel(save, lv, x[3]);
+            const int ins[2] = {L.s, L.bs};
+            ew_rows<2, 6>(tm, T, P.mt, ins, [&](int e, const vd *x) {
+                vd sv = vsel(restore, x[1], x[0]);
+                ROWD(T, L.bs + e) = vsel(save, sv, x[1]);
                 if (any_fin && P.pim)
                     sv = vsel(fin, sv * (vd(ROWD(T, L.eq + zb + e)) / ftau), sv);
                 else if (any_fin)
                     sv = vsel(fin, sv * (EI_LDG(P.GeqE + e) / ftau), sv);
                 ROWD(T, L.s + e) = sv;
-                ROWD(T, L.lam + e) = lv;
             });
         }
     }
@@ -2031,30 +2055,15 @@ EI_DEV void tile_head(const Team &tm, const KArgs &a, int tile)
     // ---- updateScalings (:411-479); its return value is ignored by the caller (:1160), so after a
     // failure at cone c the LP part and cones < c are new, cone c is partly new and lambda is stale.
     const int sz = L.w + zb; // z rows of the iterate
-    const bool lp_only = P.nc == 0; // then lambda = W z is folded into the LP pass
+    const bool lp_only = P.nc == 0; // then scale()'s lambda = W z is not stored (lp_lambda)
     if (lp_only && tm.all(cont))
     {
         const int ins[2] = {L.s, sz};
         ew_rows<2, 6>(tm, T, P.l, ins, [&](int k, const vd *x) {
             const vd v = x[0] / x[1];
-            const vd w = vsqrt(v);
             ROWD(T, L.lpv + k) = -v;
-            ROWD(T, L.lpw + k) = w;
+            ROWD(T, L.lpw + k) = vsqrt(v);
             ROWD(T, L.V + k) = -v - Settings::deltastat; // updateKKTScalings, LP part (:1696-1699)
-            ROWD(T, L.lam + k) = w * x[1];                // scale(): lambda = W z
-        });
-    }
-    else if (lp_only)
-    {
-        const int ins[5] = {L.s, sz, L.lpv, L.lpw, L.lam};
-        ew_rows<5, 2>(tm, T, P.l, ins, [&](int k, const vd *x) {
-            const vd v = x[0] / x[1];
-            const vd nvn = vsel(cont, -v, x[2]); // (lpv holds -w^2)
-            const vd wn = vsel(cont, vsqrt(v), x[3]);
-            ROWD(T, L.lpv + k) = nvn;
-            ROWD(T, L.lpw + k) = wn;
-            ROWD(T, L.V + k) = nvn - Settings::deltastat;
-            ROWD(T, L.lam + k) = vsel(cont, wn * x[1], x[4]);
         });
     }
     else
@@ -2203,19 +2212,18 @@ EI_DEV void tile_mid(const Team &tm, const KArgs &a, int tile)
     team_sum<6>(tm, dt);
     const vd dtau_denom = kap / tau - dt[0] - dt[1] - dt[2];
     const vd dtauaff = (rt - kap + dt[3] + dt[4] + dt[5]) / dtau_denom;
-    // LP rows in one pass: dz2 += dtauaff * dz1, W dz, ds = -(W dz) - lambda, min ratios of the line search
+    // LP rows in one pass: dz = dz2 + dtauaff * dz1, W dz, ds = -(W dz) - lambda, min ratios of the line search.
+    // Nothing is stored: RHScombined below recomputes the three rows, and the combined solve overwrites sol2.
+    const int lrow = lp_lambda_row(P, L);
     vd m0 = vset(DBL_MAX), m1 = vset(DBL_MAX);
     {
-        const int ins[4] = {L.sol2 + zb, L.sol1 + zb, L.lpw, L.lam};
-        ew_rows<4, 3>(tm, T, P.l, ins, [&](int k, const vd *x) {
-            const vd dz = x[0] + dtauaff * x[1];
-            const vd wd = x[2] * dz;
-            const vd ds = -wd - x[3];
-            ROWD(T, L.sol2 + zb + k) = dz;
-            ROWD(T, L.wdz + k) = wd;
-            ROWD(T, L.dsw + k) = ds;
-            m0 = vmin(m0, ds / x[3]);
-            m1 = vmin(m1, wd / x[3]);
+        const int ins[4] = {L.sol2 + zb, L.sol1 + zb, L.lpw, lrow};
+        ew_rows<4, 3>(tm, T, P.l, ins, [&](int, const vd *x) {
+            const vd lk = lp_lambda(P, x[2], x[3]);
+            const vd wd = vmul_rn(x[2], vfma(dtauaff, x[1], x[0]));
+            const vd ds = -wd - lk;
+            m0 = vmin(m0, ds / lk);
+            m1 = vmin(m1, wd / lk);
         });
     }
     if (P.mt > P.l)
@@ -2263,11 +2271,13 @@ EI_DEV void tile_mid(const Team &tm, const KArgs &a, int tile)
             ROWD(T, L.rhs2 + r) = v;
             mx[0] = vmax(mx[0], vabs(v));
         });
-        const int inl[5] = {L.lam, L.dsw, L.wdz, L.r + zb, L.lpw};
+        const int inl[5] = {lrow, L.sol2 + zb, L.sol1 + zb, L.r + zb, L.lpw};
         ew_rows<5, 2>(tm, T, P.l, inl, [&](int k, const vd *x) {
-            const vd lk = x[0];
+            const vd lk = lp_lambda(P, x[4], x[0]);
+            const vd wd = vmul_rn(x[4], vfma(dtauaff, x[2], x[1])); // the affine pass's W dz and ds
+            const vd ds = -wd - lk;
             vd d1 = lk * lk;
-            d1 += x[1] * x[2];
+            d1 += ds * wd;
             d1 -= sigmamu;
             const vd q = d1 / lk; // conicDivision, LP part
             ROWD(T, L.dsw + k) = q;
@@ -2374,22 +2384,17 @@ EI_DEV void tile_tail(const Team &tm, const KArgs &a, int tile)
     team_sum<3>(tm, dt);
     const vd bkap = kap * tau + dkapaff * dtauaff - sigma * mu;
     const vd dtau = ((1. - sigma) * rt - bkap / tau + dt[0] + dt[1] + dt[2]) / dtau_denom;
-    {
-        const int ins[2] = {L.sol2, L.sol1};
-        ew_rows<2, 6>(tm, T, zb, ins, [&](int r, const vd *x) { ROWD(T, L.sol2 + r) = x[0] + dtau * x[1]; });
-    }
-    // LP rows in one pass: dz += dtau * dz1, W dz, ds = -(ds + W dz), min ratios of the line search
+    // LP rows in one pass: dz = dz2 + dtau * dz1, W dz, ds = -(ds + W dz), min ratios of the line search.
+    // Nothing is stored: the update pass below recomputes dz and ds (and dx, dy) in registers.
     vd m0 = vset(DBL_MAX), m1 = vset(DBL_MAX);
     {
-        const int ins[5] = {L.sol2 + zb, L.sol1 + zb, L.lpw, L.dsw, L.lam};
-        ew_rows<5, 2>(tm, T, P.l, ins, [&](int k, const vd *x) {
-            const vd dz = x[0] + dtau * x[1];
-            const vd wd = x[2] * dz;
+        const int ins[5] = {L.sol2 + zb, L.sol1 + zb, L.lpw, L.dsw, lp_lambda_row(P, L)};
+        ew_rows<5, 2>(tm, T, P.l, ins, [&](int, const vd *x) {
+            const vd lk = lp_lambda(P, x[2], x[4]);
+            const vd wd = vmul_rn(x[2], vfma(dtau, x[1], x[0]));
             const vd ds = -(x[3] + wd);
-            ROWD(T, L.sol2 + zb + k) = dz;
-            ROWD(T, L.dsw + k) = ds;
-            m0 = vmin(m0, ds / x[4]);
-            m1 = vmin(m1, wd / x[4]);
+            m0 = vmin(m0, ds / lk);
+            m1 = vmin(m1, wd / lk);
         });
     }
     if (P.mt > P.l)
@@ -2412,13 +2417,16 @@ EI_DEV void tile_tail(const Team &tm, const KArgs &a, int tile)
         tm.sync();
     }
     {
-        const int ins[2] = {L.w, L.sol2};
-        ew_rows<2, 6>(tm, T, zb, ins, [&](int q, const vd *x) { ROWD(T, L.w + q) = vsel(act, x[0] + step * x[1], x[0]); });
-        // LP rows: z += step * dz and s += step * (W ds) in one pass
-        const int inl[5] = {L.w + zb, L.sol2 + zb, L.s, L.lpw, L.dsw};
-        ew_rows<5, 2>(tm, T, P.l, inl, [&](int k, const vd *x) {
-            ROWD(T, L.w + zb + k) = vsel(act, x[0] + step * x[1], x[0]);
-            ROWD(T, L.s + k) = vsel(act, x[2] + step * (x[3] * x[4]), x[2]);
+        // x, y += step * (dxy2 + dtau * dxy1)
+        const int ins[3] = {L.w, L.sol2, L.sol1};
+        ew_rows<3, 4>(tm, T, zb, ins, [&](int q, const vd *x) { ROWD(T, L.w + q) = vsel(act, x[0] + step * (x[1] + dtau * x[2]), x[0]); });
+        // LP rows: z += step * dz and s += step * (W ds) in one pass, dz and ds as in the pass before the line search
+        const int inl[6] = {L.w + zb, L.sol2 + zb, L.sol1 + zb, L.s, L.lpw, L.dsw};
+        ew_rows<6, 2>(tm, T, P.l, inl, [&](int k, const vd *x) {
+            const vd dz = vfma(dtau, x[2], x[1]);
+            const vd ds = -(x[5] + vmul_rn(x[4], dz));
+            ROWD(T, L.w + zb + k) = vsel(act, vfma(step, dz, x[0]), x[0]);
+            ROWD(T, L.s + k) = vsel(act, vfma(step, vmul_rn(x[4], ds), x[3]), x[3]);
         });
     }
     for (int c = tm.wk; c < P.nc; c += tm.nwk)
