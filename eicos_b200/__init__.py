@@ -4,4 +4,4 @@ Only the hot path of EmbersArc/EiCOS is here (Solver construction -> solve -> up
 solution, plus a batched overload); see DESIGN.md.  The compute path is hand-written CUDA for
 sm_100a in eicos_b200/csrc, reached through the C ABI in include/eicos_b200.h.
 """
-from .binding import BatchSolver, Library, MultiBatchSolver, Solver, load, PRODUCT_LIB, EXPORTS  # noqa: F401
+from .binding import BatchSolver, Library, MultiBatchSolver, Settings, Solver, default_settings, load, PRODUCT_LIB, EXPORTS  # noqa: F401

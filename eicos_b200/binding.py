@@ -30,6 +30,44 @@ class Info(C.Structure):
         return {k: getattr(self, k) for k, _ in self._fields_}
 
 
+class Settings(C.Structure):
+    """eicos_settings: the solver settings a handle applies to every later solve (include/eicos_b200.h)."""
+    _fields_ = [(k, C.c_double) for k in
+                ("feastol", "abstol", "reltol", "feastol_inacc", "abstol_inacc", "reltol_inacc",
+                 "linsysacc", "irerrfact", "gamma", "stepmin", "stepmax", "sigmamin", "sigmamax", "safeguard")] + \
+               [(k, C.c_int) for k in ("nitref", "iter_max")]
+
+    def asdict(self):
+        return {k: getattr(self, k) for k, _ in self._fields_}
+
+
+class _HasSettings:
+    """settings() / set_settings(**fields) over the handle's get / set functions (_GET, _SET)."""
+
+    def settings(self):
+        """The handle's solver settings as a dict (the keys of eicos_settings)."""
+        st = Settings()
+        self.lib.check(getattr(self.lib.L, self._GET)(self.h, C.byref(st)))
+        return st.asdict()
+
+    def set_settings(self, **fields):
+        """Merge `fields` into the current settings; every later solve uses them.  An unknown key raises
+        ValueError; a value out of range raises RuntimeError naming the field and changes nothing."""
+        cur = self.settings()
+        unknown = sorted(set(fields) - set(cur))
+        if unknown:
+            raise ValueError(f"unknown solver settings: {', '.join(unknown)} (known: {', '.join(cur)})")
+        cur.update(fields)
+        self.lib.check(getattr(self.lib.L, self._SET)(self.h, C.byref(Settings(**cur))))
+
+
+def default_settings(lib=None):
+    """The reference's default settings (eicos_default_settings) as a dict."""
+    st = Settings()
+    (lib or load()).L.eicos_default_settings(C.byref(st))
+    return st.asdict()
+
+
 class BatchStats(C.Structure):
     _fields_ = [("chunks", C.c_int), ("ipm_iterations", C.c_int), ("launches", C.c_longlong),
                 ("ir_rounds", C.c_ulonglong), ("ms_total", C.c_double), ("ms_factor", C.c_double),
@@ -69,6 +107,8 @@ class ProgramStats(C.Structure):
 EXPORTS = [
     "eicos_setup", "eicos_update_data", "eicos_update_data_full", "eicos_solve", "eicos_solution",
     "eicos_get_duals", "eicos_get_info", "eicos_cleanup",
+    "eicos_default_settings", "eicos_set_settings", "eicos_get_settings",
+    "eicos_batch_set_settings", "eicos_batch_get_settings", "eicos_multi_set_settings", "eicos_multi_get_settings",
     "eicos_batch_setup", "eicos_batch_setup_ex", "eicos_batch_update_matrices", "eicos_batch_solve",
     "eicos_batch_solve_matrices", "eicos_batch_solve_device", "eicos_batch_solve_matrices_device",
     "eicos_batch_set_timing", "eicos_batch_set_compaction", "eicos_batch_get_stats", "eicos_batch_get_dims", "eicos_batch_get_program_stats", "eicos_batch_get_symbolic",
@@ -167,6 +207,13 @@ class Library:
         L.eicos_last_error.argtypes = []
         L.eicos_device_count.restype = C.c_int
         L.eicos_device_count.argtypes = []
+        L.eicos_default_settings.restype = None
+        L.eicos_default_settings.argtypes = [C.POINTER(Settings)]
+        for kind in ("", "batch_", "multi_"):
+            getattr(L, f"eicos_{kind}set_settings").restype = C.c_int
+            getattr(L, f"eicos_{kind}set_settings").argtypes = [C.c_void_p, C.POINTER(Settings)]
+            getattr(L, f"eicos_{kind}get_settings").restype = C.c_int
+            getattr(L, f"eicos_{kind}get_settings").argtypes = [C.c_void_p, C.POINTER(Settings)]
 
     def last_error(self):
         return (self.L.eicos_last_error() or b"").decode()
@@ -203,9 +250,11 @@ def _problem_args(P):
     return keep, args, (n, m if Gpr is not None else 0, p if Apr is not None else 0)
 
 
-class Solver:
+class Solver(_HasSettings):
     """Single-instance solver; same call sequence as EiCOS::Solver / the ECOS shim
     (reference test/ecos.h:11-34): Solver(problem) -> solve() -> update_data(...) -> solve()."""
+
+    _GET, _SET = "eicos_get_settings", "eicos_set_settings"
 
     def __init__(self, problem, device=0, lib=None):
         self.lib = lib or load()
@@ -248,9 +297,11 @@ class Solver:
         return i.asdict()
 
 
-class BatchSolver:
+class BatchSolver(_HasSettings):
     """Batched overload: one pattern + shared G/A values, stacked per-instance c/h/b.
     instance_matrices=True: instances may also bring their own G/A values (solve(..., Gs=, As=))."""
+
+    _GET, _SET = "eicos_batch_get_settings", "eicos_batch_set_settings"
 
     INSTANCE_MATRICES = 1
 
@@ -302,7 +353,8 @@ class BatchSolver:
         self.lib.check(self.lib.L.eicos_batch_set_timing(self.h, int(on)))
 
     def debug_set_iter_max(self, iter_max):
-        """Test hook: cap the interior-point iterations (0 = the reference's 100)."""
+        """Test hook: cap the interior-point iterations at min(iter_max, 100) (0 = the reference's 100); the cap is
+        settings()["iter_max"]."""
         self.lib.check(self.lib.L.eicos_batch_debug_set_iter_max(self.h, int(iter_max)))
 
     def set_compaction(self, on=True):
@@ -361,9 +413,11 @@ class BatchSolver:
         return dict(Lx=Lx, D=D, sol1=s1, sol2=s2, nitref=nit)
 
 
-class MultiBatchSolver:
+class MultiBatchSolver(_HasSettings):
     """The batched overload over several GPUs of one node (eicos_multi_*): contiguous slices of the batch, one
     device and one host thread each, results gathered into the caller's arrays; no collective."""
+
+    _GET, _SET = "eicos_multi_get_settings", "eicos_multi_set_settings"
 
     def __init__(self, problem, devices=(0,), capacity=0, workers=0, lib=None, instance_matrices=False):
         self.lib = lib or load()

@@ -6,6 +6,7 @@
 #include "symbolic.hpp"
 
 #include <algorithm>
+#include <cmath>
 #include <cstring>
 #include <memory>
 #include <thread>
@@ -24,7 +25,7 @@ int fail(int code, const std::string &msg)
     return code;
 }
 
-void info_from_rows(const double *d, const int *i, eicos_info *o)
+void info_from_rows(const double *d, const int *i, int iter_max, eicos_info *o)
 {
     o->pcost = d[S_PCOST];
     o->dcost = d[S_DCOST];
@@ -45,10 +46,64 @@ void info_from_rows(const double *d, const int *i, eicos_info *o)
     o->has_dinfres = i[J_HAS_DINFRES];
     o->has_relgap = i[J_HAS_RELGAP];
     o->iter = i[J_ITER];
-    o->iter_max = Settings::iter_max;
+    o->iter_max = iter_max;
     o->nitref1 = i[J_NIT1];
     o->nitref2 = i[J_NIT2];
     o->nitref3 = i[J_NIT3];
+}
+
+// eicos_settings <-> KSettings: the same fields under the same names
+#define EICOS_SETTINGS_FIELDS(X)                                                                                       \
+    X(feastol) X(abstol) X(reltol) X(feastol_inacc) X(abstol_inacc) X(reltol_inacc) X(linsysacc) X(irerrfact)         \
+        X(gamma) X(stepmin) X(stepmax) X(sigmamin) X(sigmamax) X(safeguard) X(nitref) X(iter_max)
+
+void settings_out(const KSettings &k, eicos_settings *o)
+{
+#define EICOS_COPY(f) o->f = k.f;
+    EICOS_SETTINGS_FIELDS(EICOS_COPY)
+#undef EICOS_COPY
+}
+
+// Checks every field; on success fills *k and returns 0, otherwise fails naming the first bad field.
+int settings_in(const eicos_settings *s, KSettings *k)
+{
+    if (!s)
+        return fail(EICOS_ERR_INVALID, "null settings");
+    const auto bad = [](const char *field, const char *rule) {
+        return fail(EICOS_ERR_INVALID, std::string("eicos_settings.") + field + ": must be " + rule);
+    };
+#define EICOS_FINITE(f)                                                                                               \
+    if (!std::isfinite((double)s->f))                                                                                  \
+        return bad(#f, "finite");
+    EICOS_SETTINGS_FIELDS(EICOS_FINITE)
+#undef EICOS_FINITE
+#define EICOS_POSITIVE(f)                                                                                             \
+    if (!(s->f > 0.))                                                                                                  \
+        return bad(#f, "> 0");
+    EICOS_POSITIVE(feastol) EICOS_POSITIVE(abstol) EICOS_POSITIVE(reltol)
+    EICOS_POSITIVE(feastol_inacc) EICOS_POSITIVE(abstol_inacc) EICOS_POSITIVE(reltol_inacc)
+    EICOS_POSITIVE(linsysacc) EICOS_POSITIVE(irerrfact)
+#undef EICOS_POSITIVE
+    if (!(s->gamma > 0. && s->gamma <= 1.))
+        return bad("gamma", "in (0, 1]");
+    if (!(s->stepmin > 0. && s->stepmin <= s->stepmax))
+        return bad("stepmin", "in (0, stepmax]");
+    if (!(s->stepmax <= 1.))
+        return bad("stepmax", "<= 1");
+    if (!(s->sigmamin >= 0. && s->sigmamin <= s->sigmamax))
+        return bad("sigmamin", "in [0, sigmamax]");
+    if (!(s->sigmamax <= 1.))
+        return bad("sigmamax", "<= 1");
+    if (!(s->safeguard >= 1.))
+        return bad("safeguard", ">= 1");
+    if (s->nitref < 0 || s->nitref > 32)
+        return bad("nitref", "in [0, 32]");
+    if (s->iter_max < 1 || s->iter_max > 1000)
+        return bad("iter_max", "in [1, 1000]");
+#define EICOS_COPY(f) k->f = s->f;
+    EICOS_SETTINGS_FIELDS(EICOS_COPY)
+#undef EICOS_COPY
+    return 0;
 }
 
 struct DeviceBuffer
@@ -105,6 +160,12 @@ extern "C"
 {
 
 const char *eicos_last_error(void) { return g_error.c_str(); }
+
+void eicos_default_settings(eicos_settings *out)
+{
+    if (out)
+        settings_out(default_settings(), out);
+}
 
 int eicos_device_count(void)
 {
@@ -320,7 +381,7 @@ int eicos_batch_solve_matrices(eicos_batch *bt, int batch, const double *Gs, con
                 std::copy(hexit.begin(), hexit.end(), exitflag + first);
             if (info)
                 for (size_t k = 0; k < B; k++)
-                    info_from_rows(hinfo.data() + k * S_WORK_END, hii.data() + k * J_WORK_END, info + first + k);
+                    info_from_rows(hinfo.data() + k * S_WORK_END, hii.data() + k * J_WORK_END, bt->eng->settings().iter_max, info + first + k);
             total += bt->stats;
             if (batch == 0)
                 break;
@@ -507,7 +568,28 @@ int eicos_batch_debug_set_iter_max(eicos_batch *bt, int iter_max)
 {
     if (!bt)
         return fail(EICOS_ERR_INVALID, "null handle");
-    bt->eng->set_iter_max(iter_max > 0 ? std::min(iter_max, (int)Settings::iter_max) : (int)Settings::iter_max);
+    KSettings k = bt->eng->settings();
+    k.iter_max = iter_max > 0 ? std::min(iter_max, (int)Settings::iter_max) : (int)Settings::iter_max;
+    bt->eng->set_settings(k);
+    return 0;
+}
+
+int eicos_batch_set_settings(eicos_batch *bt, const eicos_settings *settings)
+{
+    if (!bt)
+        return fail(EICOS_ERR_INVALID, "null handle");
+    KSettings k;
+    if (const int rc = settings_in(settings, &k))
+        return rc;
+    bt->eng->set_settings(k);
+    return 0;
+}
+
+int eicos_batch_get_settings(const eicos_batch *bt, eicos_settings *out)
+{
+    if (!bt || !out)
+        return fail(EICOS_ERR_INVALID, "null argument");
+    settings_out(bt->eng->settings(), out);
     return 0;
 }
 
@@ -605,6 +687,26 @@ int eicos_multi_solve(eicos_multi *mt, int batch, const double *Gs, const double
     for (int k = 0; k < parts; k++)
         if (rc[k] != 0)
             return fail(rc[k], ("device slice " + std::to_string(k) + ": " + err[k]).c_str());
+    return 0;
+}
+
+int eicos_multi_set_settings(eicos_multi *mt, const eicos_settings *settings)
+{
+    if (!mt)
+        return fail(EICOS_ERR_INVALID, "null handle");
+    KSettings k;
+    if (const int rc = settings_in(settings, &k))
+        return rc;
+    for (eicos_batch *bt : mt->part)
+        bt->eng->set_settings(k);
+    return 0;
+}
+
+int eicos_multi_get_settings(const eicos_multi *mt, eicos_settings *out)
+{
+    if (!mt || !out)
+        return fail(EICOS_ERR_INVALID, "null argument");
+    settings_out(mt->part[0]->eng->settings(), out);
     return 0;
 }
 
@@ -755,6 +857,25 @@ int eicos_update_data_full(eicos_solver *s, const double *Gpr, const double *Apr
     return update_common(s, true, Gpr, Apr, c, h, b);
 }
 
+int eicos_set_settings(eicos_solver *s, const eicos_settings *settings)
+{
+    if (!s)
+        return fail(EICOS_ERR_INVALID, "null handle");
+    KSettings k;
+    if (const int rc = settings_in(settings, &k))
+        return rc;
+    s->eng->set_settings(k);
+    return 0;
+}
+
+int eicos_get_settings(const eicos_solver *s, eicos_settings *out)
+{
+    if (!s || !out)
+        return fail(EICOS_ERR_INVALID, "null argument");
+    settings_out(s->eng->settings(), out);
+    return 0;
+}
+
 int eicos_solve(eicos_solver *s)
 {
     if (!s)
@@ -781,7 +902,7 @@ int eicos_solve(eicos_solver *s)
         be::d2h(hinfo, dinfo, sizeof(hinfo), st);
         be::d2h(hi, dexit, sizeof(hi), st);
         be::sync(st);
-        info_from_rows(hinfo, hi + 1, &s->info);
+        info_from_rows(hinfo, hi + 1, s->eng->settings().iter_max, &s->info);
         return hi[0];
     }
     catch (const std::exception &e)

@@ -532,6 +532,7 @@ void Engine::debug_line_search(int batch, const double *h_lambda, const double *
     a.L = L_;
     a.ws = ws_;
     a.iws = iws_;
+    a.settings = settings_;
     a.batch = batch;
     a.in_h = d;
     a.in_G = d + zm;
@@ -585,6 +586,7 @@ void Engine::solve(int batch, const double *d_c, const double *d_h, const double
     a.L = L_;
     a.ws = ws_;
     a.iws = iws_;
+    a.settings = settings_;
     a.in_c = d_c;
     a.in_h = d_h;
     a.in_b = d_b;
@@ -613,7 +615,6 @@ void Engine::solve(int batch, const double *d_c, const double *d_h, const double
     a.out_info = d_info;
     a.out_iinfo = d_iinfo;
     a.keep_sticky = keep_sticky ? 1 : 0;
-    a.iter_max = iter_max_;
     a.pre_equilibrated = pre_equilibrated ? 1 : 0;
     a.active_count = active_count_;
     a.ir_rounds = ir_rounds_;
@@ -741,7 +742,7 @@ void Engine::solve(int batch, const double *d_c, const double *d_h, const double
         kkt_pair(1, J_NIT1, J_NIT2);
         EI_TIMED(2, EI_LAUNCH(eicos_init_point, tile_init_point, tiles, threads, smem_common_, st, a));
 
-        for (int it = 0; it <= iter_max_ + 1; it++)
+        for (int it = 0; it <= settings_.iter_max + 1; it++)
         {
             be::zero(active_count_, sizeof(unsigned int), st);
             if (wide_launch(tiles))
@@ -866,6 +867,7 @@ void Engine::debug_factor_init(int batch, const double *d_c, const double *d_h, 
     a.L = L_;
     a.ws = ws_;
     a.iws = iws_;
+    a.settings = settings_;
     a.in_c = d_c;
     a.in_h = d_h;
     a.in_b = d_b;

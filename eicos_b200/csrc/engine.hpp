@@ -99,7 +99,10 @@ class Engine
     int device() const { return device_; }
     int workers() const { return workers_; }
     void set_compaction(bool on) { compaction_ = on; }
-    void set_iter_max(int k) { iter_max_ = k; } // (test hook: eicos_batch_debug_set_iter_max)
+    // solver settings of every later solve (tolerances, iteration limit, refinement, step control); the caller
+    // validates them (capi.cu)
+    void set_settings(const KSettings &k) { settings_ = k; }
+    const KSettings &settings() const { return settings_; }
     long long capacity() const { return cap_tiles_ * (long long)tile_width(); }
     size_t workspace_bytes() const { return ws_bytes_; }
     const Layout &layout() const { return L_; }
@@ -131,7 +134,7 @@ class Engine
     size_t smem_pair_ = 0; // two-job solveKKT kernel
     size_t smem_resid_ = 0, smem_wide_ = 0, part_doubles_ = 0; // one-warp residual kernel; wide kernels; one part machine (doubles)
     int force_wide_ = -1;
-    int iter_max_ = Settings::iter_max;
+    KSettings settings_ = default_settings();
     bool wide_launch(int ctas) const;
     int sms_ = 148, force_variant_ = -1, force_pair_ = -1;
     bool deep_ring(int ctas) const;

@@ -20,7 +20,9 @@ namespace eicos
 typedef std::vector<int> ivec;
 typedef std::vector<double> dvec;
 
-// Tunable constants of the reference (include/eicos.hpp:23-47); all compile-time there as well.
+// Tunable constants of the reference (include/eicos.hpp:23-47); all compile-time there as well.  Here they are
+// the defaults of KSettings, except deltastat and equil_iters, which enter the shared KKT values, the programs'
+// constants and the equilibration at setup and so stay fixed for the life of a handle.
 struct Settings
 {
     static constexpr double gamma = 0.99, deltastat = 7e-8;
@@ -30,6 +32,32 @@ struct Settings
     static constexpr double linsysacc = 1e-14, irerrfact = 6, stepmin = 1e-6, stepmax = 0.999;
     static constexpr double sigmamin = 1e-4, sigmamax = 1.0, safeguard = 500;
 };
+
+// The settings the kernels read at run time (KArgs::settings), one set per handle.  Plain doubles and ints:
+// passed inside the __grid_constant__ KArgs, every field is read from the constant bank.
+struct KSettings
+{
+    double feastol, abstol, reltol;
+    double feastol_inacc, abstol_inacc, reltol_inacc;
+    double linsysacc, irerrfact;
+    double gamma, stepmin, stepmax;
+    double sigmamin, sigmamax;
+    double safeguard;
+    int nitref, iter_max;
+};
+
+inline KSettings default_settings()
+{
+    KSettings k;
+    k.feastol = Settings::feastol, k.abstol = Settings::abstol, k.reltol = Settings::reltol;
+    k.feastol_inacc = Settings::feastol_inacc, k.abstol_inacc = Settings::abstol_inacc, k.reltol_inacc = Settings::reltol_inacc;
+    k.linsysacc = Settings::linsysacc, k.irerrfact = Settings::irerrfact;
+    k.gamma = Settings::gamma, k.stepmin = Settings::stepmin, k.stepmax = Settings::stepmax;
+    k.sigmamin = Settings::sigmamin, k.sigmamax = Settings::sigmamax;
+    k.safeguard = Settings::safeguard;
+    k.nitref = Settings::nitref, k.iter_max = Settings::iter_max;
+    return k;
+}
 
 struct Csc
 {

@@ -222,7 +222,7 @@ struct KArgs
     int variant; // which ring depth of the programs this launch runs (streams.hpp: M_VARIANT_GROUPS)
     int part_doubles; // wide launches: shared memory (doubles) of one warp's machine
     int keep_sticky;
-    int iter_max; // Settings::iter_max, or the test hook's cap
+    KSettings settings; // the handle's solver settings (tolerances, iteration limit, refinement, step control)
     int pre_equilibrated; // inputs are already divided by the equilibration vectors
     unsigned int *active_count; // device counter: instances still iterating after the head step
     unsigned long long *ir_rounds; // device counters: [0] solve rounds executed (tile-rounds), [1..5] cycles per solve_kkt phase
@@ -519,10 +519,10 @@ EI_DEV vd line_search(const Team &tm, const KArgs &a, double *T, int lam, int ds
             alpha = mk;
         alpha = dmin(mn[2].v[c_], alpha);
         // std::clamp(alpha, stepmin, stepmax)
-        if (alpha < Settings::stepmin)
-            alpha = Settings::stepmin;
-        else if (Settings::stepmax < alpha)
-            alpha = Settings::stepmax;
+        if (alpha < a.settings.stepmin)
+            alpha = a.settings.stepmin;
+        else if (a.settings.stepmax < alpha)
+            alpha = a.settings.stepmax;
         res.v[c_] = alpha;
     }
     return res;
@@ -1293,7 +1293,7 @@ EI_DEV void tile_solve_kkt(const Team &tm, const KArgs &a, int tile)
         dxr[j] = set ? L.dxr2 : L.dxr;
         erow[j] = set ? L.e2 : L.e;
         // max |rhs| is kept up to date by the kernels that write the right-hand sides (src/eicos.cpp:1590)
-        threshold[j] = (1. + vd(ROWD(T, L.sc + (set ? S_RHSMAX2 : S_RHSMAX1)))) * Settings::linsysacc;
+        threshold[j] = (1. + vd(ROWD(T, L.sc + (set ? S_RHSMAX2 : S_RHSMAX1)))) * a.settings.linsysacc;
     }
     const int set0 = a.job[NR == 1 ? tm.job : 0].set, v = a.variant;
     // programs and load lists of this launch: [first solve | refinement round]
@@ -1392,8 +1392,8 @@ EI_DEV void tile_solve_kkt(const Team &tm, const KArgs &a, int tile)
                     kref[j][c_]--;
                     done[j].v[c_] = true;
                 }
-                else if (kref[j][c_] == Settings::nitref || nerr[j].v[c_] < threshold[j].v[c_] ||
-                         (kref[j][c_] > 0 && nerr_prev[j].v[c_] < Settings::irerrfact * nerr[j].v[c_]))
+                else if (kref[j][c_] == a.settings.nitref || nerr[j].v[c_] < threshold[j].v[c_] ||
+                         (kref[j][c_] > 0 && nerr_prev[j].v[c_] < a.settings.irerrfact * nerr[j].v[c_]))
                     done[j].v[c_] = true;
                 else
                     nerr_prev[j].v[c_] = nerr[j].v[c_];
@@ -1533,7 +1533,7 @@ EI_DEV void tile_init(const Team &tm, const KArgs &a, int tile)
 EI_DEV void bring_to_cone(const Team &tm, const KArgs &a, double *T, int src, double sign, int dst, vb write)
 {
     const DevPattern &P = a.P;
-    vd al[1] = {vset(-Settings::gamma)};
+    vd al[1] = {vset(-a.settings.gamma)};
     for (int k = tm.wk; k < P.l; k += tm.nwk)
     {
         const vd r = sign * vd(ROWD(T, src + k));
@@ -1640,11 +1640,11 @@ EI_DEV bool ws_better(const WState &a, const WState &o)
 
 // checkExitConditions (src/eicos.cpp:526-641).  An empty std::optional compares "less than"
 // any double there, which is what the (!has || v < tol) terms reproduce.
-EI_DEV int ws_check_exit(WState &w, bool reduced)
+EI_DEV int ws_check_exit(const KSettings &st, WState &w, bool reduced)
 {
-    const double feastol = reduced ? Settings::feastol_inacc : Settings::feastol;
-    const double abstol = reduced ? Settings::abstol_inacc : Settings::abstol;
-    const double reltol = reduced ? Settings::reltol_inacc : Settings::reltol;
+    const double feastol = reduced ? st.feastol_inacc : st.feastol;
+    const double abstol = reduced ? st.abstol_inacc : st.abstol;
+    const double reltol = reduced ? st.reltol_inacc : st.reltol;
     const double tau = w.d[S_TAU], kap = w.d[S_KAP];
     if ((-w.d[S_CX] > 0. || -w.d[S_BY] - w.d[S_HZ] >= -abstol) &&
         (w.d[S_PRES] < feastol && w.d[S_DRES] < feastol) &&
@@ -1900,12 +1900,12 @@ EI_DEV void tile_head(const Team &tm, const KArgs &a, int tile)
         const double nrz = sqrt(r[RZ2].v[c]) / dmax(resz0 + nx + ns, 1.);
         w.d[S_PRES] = dmax(nry, nrz) / tau_c;
         w.d[S_DRES] = sqrt(r[RX2].v[c]) / dmax(resx0 + ny + nz, 1.) / tau_c;
-        if ((hz + by) / dmax(ny + nz, 1.) < -Settings::reltol)
+        if ((hz + by) / dmax(ny + nz, 1.) < -a.settings.reltol)
         {
             w.i[J_HAS_PINFRES] = 1;
             w.d[S_PINFRES] = hresx / dmax(ny + nz, 1.);
         }
-        if (cx / dmax(nx, 1.) < -Settings::reltol)
+        if (cx / dmax(nx, 1.) < -a.settings.reltol)
         {
             w.i[J_HAS_DINFRES] = 1;
             w.d[S_DINFRES] = dmax(hresy / dmax(nx, 1.), hresz / dmax(nx + ns, 1.));
@@ -1917,36 +1917,36 @@ EI_DEV void tile_head(const Team &tm, const KArgs &a, int tile)
         bool rst = false, sav = false;
         if (act.v[c])
         {
-            if (iter > 0 && (w.d[S_PRES] > Settings::safeguard * pres_prev || w.d[S_GAP] < 0.))
+            if (iter > 0 && (w.d[S_PRES] > a.settings.safeguard * pres_prev || w.d[S_GAP] < 0.))
             {
                 rst = true;
                 w = best;
-                code = ws_check_exit(w, true);
+                code = ws_check_exit(a.settings, w, true);
                 if (code == EXIT_NOT_CONVERGED)
                     code = EXIT_NUMERICS;
             }
             else
             {
                 pres_prev = w.d[S_PRES];
-                code = ws_check_exit(w, false);
+                code = ws_check_exit(a.settings, w, false);
                 if (code == EXIT_NOT_CONVERGED)
                 {
-                    if (iter > 0 && w.d[S_STEP] == Settings::stepmin * Settings::gamma)
+                    if (iter > 0 && w.d[S_STEP] == a.settings.stepmin * a.settings.gamma)
                     {
                         rst = true;
                         w = best;
-                        code = ws_check_exit(w, true);
+                        code = ws_check_exit(a.settings, w, true);
                         if (code == EXIT_NOT_CONVERGED)
                             code = EXIT_NUMERICS;
                     }
-                    else if (iter == a.iter_max)
+                    else if (iter == a.settings.iter_max)
                     {
                         if (!ws_better(w, best))
                         {
                             rst = true;
                             w = best;
                         }
-                        code = ws_check_exit(w, true);
+                        code = ws_check_exit(a.settings, w, true);
                         if (code == EXIT_NOT_CONVERGED)
                             code = EXIT_MAXIT;
                     }
@@ -1956,7 +1956,7 @@ EI_DEV void tile_head(const Team &tm, const KArgs &a, int tile)
                         {
                             rst = true;
                             w = best;
-                            code = ws_check_exit(w, true);
+                            code = ws_check_exit(a.settings, w, true);
                             if (code == EXIT_NOT_CONVERGED)
                                 code = EXIT_NUMERICS;
                         } // else: the reference leaves not_converged_yet (-87) in place (:1117-1121)
@@ -2245,10 +2245,10 @@ EI_DEV void tile_mid(const Team &tm, const KArgs &a, int tile)
     {
         const double om = 1. - step_aff.v[c_];
         double sg = om * om * om; // std::pow(x, 3)
-        if (sg < Settings::sigmamin)
-            sg = Settings::sigmamin;
-        else if (Settings::sigmamax < sg)
-            sg = Settings::sigmamax;
+        if (sg < a.settings.sigmamin)
+            sg = a.settings.sigmamin;
+        else if (a.settings.sigmamax < sg)
+            sg = a.settings.sigmamax;
         sigma.v[c_] = sg;
     }
     if (tm.wk == 0)
@@ -2410,7 +2410,7 @@ EI_DEV void tile_tail(const Team &tm, const KArgs &a, int tile)
         tm.sync();
     }
     const vd dkap = -(bkap + kap * dtau) / tau;
-    const vd step = Settings::gamma * line_search(tm, a, T, L.lam, L.dsw, L.wdz, tau, dtau, kap, dkap, false, m0, m1);
+    const vd step = a.settings.gamma * line_search(tm, a, T, L.lam, L.dsw, L.wdz, tau, dtau, kap, dkap, false, m0, m1);
     if (P.mt > P.l)
     {
         cone_scale(tm, a, T, L.dsw, L.dsaff, vbset(true), false);

@@ -9,8 +9,12 @@
 //  * solution() returns a pointer-backed view (VectorView) instead of `const Eigen::VectorXd &`;
 //    with Eigen present (EICOS_B200_WITH_EIGEN, set automatically when <Eigen/Sparse> is found) the
 //    Eigen-typed constructor / updateData exist and VectorView converts to Eigen::Map.
-//  * Settings are read-only: the reference declares every numeric field `const` as well
-//    (include/eicos.hpp:25-46); `verbose` is accepted and ignored (printing is out of scope).
+//  * Settings can be changed: getSettings().feastol = 1e-6 takes effect at the next solve().  The reference
+//    declares every numeric field `const` (include/eicos.hpp:25-46); here the tolerances, nitref, iter_max and
+//    the step and centering controls are writable and checked when solve() hands them to the engine (an
+//    out-of-range value throws std::runtime_error naming the field).  deltastat and equil_iters stay `const`:
+//    they are baked into a handle at setup.  delta, eps and maxit are not read (the reference does not read them
+//    either); `verbose` is accepted and ignored (printing is out of scope).
 //  * getInfo() carries the scalar fields of Information; the iterate vectors are reached through
 //    solution() / duals().
 #pragma once
@@ -50,31 +54,47 @@ enum class exitcode
     not_converged_yet = -87
 };
 
-// reference include/eicos.hpp:23-47.  The engine compiles these values in (csrc/layout.hpp: Settings).
+// reference include/eicos.hpp:23-47, same defaults.  The writable fields go to the engine before every solve
+// (eicos_settings); the const ones are fixed at setup (deltastat, equil_iters) or unused (delta, eps, maxit).
 struct Settings
 {
-    const double gamma = 0.99;
+    double gamma = 0.99;
     const double delta = 2e-7;
     const double deltastat = 7e-8;
     const double eps = 1e13;
-    const double feastol = 1e-8;
-    const double abstol = 1e-8;
-    const double reltol = 1e-8;
-    const double feastol_inacc = 1e-4;
-    const double abstol_inacc = 5e-5;
-    const double reltol_inacc = 5e-5;
-    const size_t nitref = 9;
+    double feastol = 1e-8;
+    double abstol = 1e-8;
+    double reltol = 1e-8;
+    double feastol_inacc = 1e-4;
+    double abstol_inacc = 5e-5;
+    double reltol_inacc = 5e-5;
+    size_t nitref = 9;
     const size_t maxit = 100;
     bool verbose = false;
-    const double linsysacc = 1e-14;
-    const double irerrfact = 6;
-    const double stepmin = 1e-6;
-    const double stepmax = 0.999;
-    const double sigmamin = 1e-4;
-    const double sigmamax = 1.;
+    double linsysacc = 1e-14;
+    double irerrfact = 6;
+    double stepmin = 1e-6;
+    double stepmax = 0.999;
+    double sigmamin = 1e-4;
+    double sigmamax = 1.;
     const size_t equil_iters = 3;
-    const size_t iter_max = 100;
-    const size_t safeguard = 500;
+    size_t iter_max = 100;
+    size_t safeguard = 500;
+
+    // the engine's form (values past INT_MAX saturate, so that the range check rejects them)
+    eicos_settings to_c() const
+    {
+        const auto narrow = [](size_t v) { return v > 0x7fffffff ? 0x7fffffff : (int)v; };
+        eicos_settings o;
+        o.feastol = feastol, o.abstol = abstol, o.reltol = reltol;
+        o.feastol_inacc = feastol_inacc, o.abstol_inacc = abstol_inacc, o.reltol_inacc = reltol_inacc;
+        o.linsysacc = linsysacc, o.irerrfact = irerrfact;
+        o.gamma = gamma, o.stepmin = stepmin, o.stepmax = stepmax;
+        o.sigmamin = sigmamin, o.sigmamax = sigmamax;
+        o.safeguard = (double)safeguard;
+        o.nitref = narrow(nitref), o.iter_max = narrow(iter_max);
+        return o;
+    }
 };
 
 // reference include/eicos.hpp:49-73
@@ -186,12 +206,14 @@ class Solver
     ~Solver() { eicos_cleanup(h_); }
     Solver(const Solver &) = delete;
     Solver &operator=(const Solver &) = delete;
-    Solver(Solver &&o) noexcept : h_(o.h_), n_(o.n_), m_(o.m_), p_(o.p_) { o.h_ = nullptr; }
+    Solver(Solver &&o) noexcept : h_(o.h_), n_(o.n_), m_(o.m_), p_(o.p_), settings_(o.settings_) { o.h_ = nullptr; }
 
-    // reference include/eicos.hpp:158
+    // reference include/eicos.hpp:158; runs with the current getSettings()
     exitcode solve(bool verbose = false)
     {
         (void)verbose;
+        const eicos_settings st = settings_.to_c();
+        detail::check(eicos_set_settings(h_, &st), "EiCOS::Solver::solve");
         const int rc = eicos_solve(h_);
         if (rc <= EICOS_ERR_INVALID)
             throw std::runtime_error(std::string("EiCOS::Solver::solve: ") + eicos_last_error());
@@ -297,12 +319,16 @@ class BatchSolver
             r.info.resize(B);
         double *y = want_duals ? r.y.data() : nullptr, *z = want_duals ? r.z.data() : nullptr, *s = want_duals ? r.s.data() : nullptr;
         eicos_info *info = want_info ? r.info.data() : nullptr;
+        const eicos_settings st = settings_.to_c();
+        detail::check(mh_ ? eicos_multi_set_settings(mh_, &st) : eicos_batch_set_settings(h_, &st), "EiCOS::BatchSolver::solve");
         detail::check(mh_ ? eicos_multi_solve(mh_, batch, Gs, As, cs, hs, bs, r.x.data(), y, z, s, r.exitflag.data(), info)
                           : eicos_batch_solve_matrices(h_, batch, Gs, As, cs, hs, bs, r.x.data(), y, z, s, r.exitflag.data(), info),
                       "EiCOS::BatchSolver::solve");
         return r;
     }
 
+    // settings of every instance of the next solve() (reference include/eicos.hpp:162)
+    Settings &getSettings() { return settings_; }
     int nnzG() const { return nnzG_; }
     int nnzA() const { return nnzA_; }
     eicos_batch *handle() const { return h_; }
@@ -312,6 +338,7 @@ class BatchSolver
     eicos_batch *h_ = nullptr;
     eicos_multi *mh_ = nullptr; // set instead of h_ by the multi-device constructor
     int n_ = 0, m_ = 0, p_ = 0, nnzG_ = 0, nnzA_ = 0;
+    Settings settings_;
 };
 
 } // namespace EiCOS
