@@ -111,6 +111,7 @@ EXPORTS = [
     "eicos_batch_set_settings", "eicos_batch_get_settings", "eicos_multi_set_settings", "eicos_multi_get_settings",
     "eicos_batch_setup", "eicos_batch_setup_ex", "eicos_batch_update_matrices", "eicos_batch_solve",
     "eicos_batch_solve_matrices", "eicos_batch_solve_device", "eicos_batch_solve_matrices_device",
+    "eicos_batch_adjoint", "eicos_batch_adjoint_device",
     "eicos_batch_set_timing", "eicos_batch_set_compaction", "eicos_batch_get_stats", "eicos_batch_get_dims", "eicos_batch_get_program_stats", "eicos_batch_get_symbolic",
     "eicos_batch_debug_init", "eicos_batch_debug_line_search", "eicos_batch_debug_set_iter_max", "eicos_batch_stream", "eicos_batch_cleanup",
     "eicos_multi_setup", "eicos_multi_solve", "eicos_multi_ngpu", "eicos_multi_slice", "eicos_multi_cleanup",
@@ -171,6 +172,10 @@ class Library:
         L.eicos_batch_solve_device.argtypes = [C.c_void_p, C.c_int] + [C.c_void_p] * 9
         L.eicos_batch_solve_matrices_device.restype = C.c_int
         L.eicos_batch_solve_matrices_device.argtypes = [C.c_void_p, C.c_int] + [C.c_void_p] * 11
+        L.eicos_batch_adjoint.restype = C.c_int
+        L.eicos_batch_adjoint.argtypes = [C.c_void_p, C.c_int] + [_dp] * 6 + [_ip] + [_dp] * 8 + [_ip]
+        L.eicos_batch_adjoint_device.restype = C.c_int
+        L.eicos_batch_adjoint_device.argtypes = [C.c_void_p, C.c_int] + [C.c_void_p] * 16
         L.eicos_batch_set_timing.restype = C.c_int
         L.eicos_batch_set_timing.argtypes = [C.c_void_p, C.c_int]
         L.eicos_batch_set_compaction.restype = C.c_int
@@ -307,6 +312,7 @@ class BatchSolver(_HasSettings):
 
     def __init__(self, problem, device=0, capacity=0, workers=0, lib=None, instance_matrices=False):
         self.lib = lib or load()
+        self.instance_matrices = bool(instance_matrices)
         self._keep, args, (self.n, self.m, self.p) = _problem_args(problem)
         self.h = self.lib.L.eicos_batch_setup_ex(*args, int(device), int(capacity), int(workers),
                                                  self.INSTANCE_MATRICES if instance_matrices else 0)
@@ -394,6 +400,51 @@ class BatchSolver(_HasSettings):
         """Raw device pointers (ints); results stay in HBM."""
         self.lib.check(self.lib.L.eicos_batch_solve_matrices_device(
             self.h, int(batch), *[C.c_void_p(int(v) or None) for v in (d_Gs, d_As, d_cs, d_hs, d_bs, d_x, d_y, d_z, d_s, d_exit, d_iter)]))
+
+    ADJOINT_OUTPUTS = ("c", "h", "b", "G", "A")
+
+    def adjoint(self, out, gx=None, gy=None, gz=None, Gs=None, As=None, want=ADJOINT_OUTPUTS):
+        """Gradients of L(x, y, z) with respect to the problem data of the instances `out` = solve(...) returned
+        (eicos_batch_adjoint): gx [batch x n], gy [batch x p], gz [batch x m] are dL/dx, dL/dy, dL/dz (None = zero);
+        Gs / As: the forward's per-instance matrices (instance-matrices handles only; None = the setup values).
+        Returns {"c": [batch x n], "h": [batch x m], "b": [batch x p], "G": [batch x nnzG], "A": [batch x nnzA]}
+        for the names in `want`, and "status" [batch] (0 differentiated, 1 not optimal, 2 not interior, 3 not
+        finite; instances with status != 0 get zeros)."""
+        unknown = sorted(set(want) - set(self.ADJOINT_OUTPUTS))
+        if unknown:
+            raise ValueError(f"unknown adjoint outputs: {', '.join(unknown)}")
+        batch = int(np.asarray(out["exit"]).size)
+        sizes = {"x": self.n, "y": self.p, "z": self.m, "s": self.m}
+        it = {k: np.ascontiguousarray(out[k], np.float64) for k in sizes}
+        ex = np.ascontiguousarray(out["exit"], np.int32)
+        g = {k: _arr(v, np.float64) for k, v in (("x", gx), ("y", gy), ("z", gz))}
+        Gs, As = _arr(Gs, np.float64), _arr(As, np.float64)
+        for k, a in it.items():
+            if a.size != batch * sizes[k]:
+                raise ValueError(f"out[{k!r}] has the wrong size")
+        for k, a in g.items():
+            if a is not None and a.size != batch * sizes[k]:
+                raise ValueError(f"g{k} has the wrong size")
+        for a, k in ((Gs, self.nnzG), (As, self.nnzA)):
+            if a is not None and a.size != batch * k:
+                raise ValueError("stacked matrix values have the wrong size")
+        dims = {"c": self.n, "h": self.m, "b": self.p, "G": self.nnzG, "A": self.nnzA}
+        res = {k: np.zeros((batch, dims[k])) if k in want else None for k in self.ADJOINT_OUTPUTS}
+        status = np.zeros(batch, np.int32)
+        self.lib.check(self.lib.L.eicos_batch_adjoint(
+            self.h, batch, _d(Gs), _d(As), *[_d(it[k]) for k in "xyzs"], _i(ex), _d(g["x"]), _d(g["y"]), _d(g["z"]),
+            *[_d(res[k]) for k in self.ADJOINT_OUTPUTS], _i(status)))
+        res = {k: v for k, v in res.items() if v is not None}
+        res["status"] = status
+        return res
+
+    def adjoint_device(self, batch, d_x=0, d_y=0, d_z=0, d_s=0, d_exit=0, d_gx=0, d_gy=0, d_gz=0,
+                       d_dc=0, d_dh=0, d_db=0, d_dG=0, d_dA=0, d_status=0, d_Gs=0, d_As=0):
+        """eicos_batch_adjoint_device on raw device pointers (ints, 0 = NULL); results stay in HBM."""
+        self.lib.check(self.lib.L.eicos_batch_adjoint_device(
+            self.h, int(batch), *[C.c_void_p(int(v) or None) for v in
+                                  (d_Gs, d_As, d_x, d_y, d_z, d_s, d_exit, d_gx, d_gy, d_gz,
+                                   d_dc, d_dh, d_db, d_dG, d_dA, d_status)]))
 
     def debug_line_search(self, lam, ds, dz, scalars):
         """lineSearch on caller data: lam, ds, dz [batch x m] in z order, scalars [batch x 4] = tau, dtau, kap, dkap."""

@@ -399,6 +399,114 @@ int eicos_batch_solve_matrices(eicos_batch *bt, int batch, const double *Gs, con
     }
 }
 
+static int adjoint_check(const eicos_batch *bt, int batch, const void *Gs, const void *As, const void *x, const void *y,
+                         const void *z, const void *s, const void *exitflag)
+{
+    if (!bt || batch <= 0)
+        return fail(EICOS_ERR_INVALID, "eicos_batch_adjoint: null handle or batch <= 0");
+    if ((Gs || As) && !bt->eng->instance_matrices())
+        return fail(EICOS_ERR_INVALID, "eicos_batch_adjoint: Gs / As need a handle from eicos_batch_setup_ex(..., EICOS_BATCH_INSTANCE_MATRICES)");
+    const Symbolic &S = bt->S;
+    if ((!x && S.n) || (!y && S.p) || (!z && S.m) || (!s && S.m) || !exitflag)
+        return fail(EICOS_ERR_INVALID, "eicos_batch_adjoint: x, y, z, s and exitflag are required");
+    return 0;
+}
+
+int eicos_batch_adjoint_device(eicos_batch *bt, int batch, const double *d_Gs, const double *d_As,
+                               const double *d_x, const double *d_y, const double *d_z, const double *d_s,
+                               const int *d_exitflag, const double *d_gx, const double *d_gy, const double *d_gz,
+                               double *d_dc, double *d_dh, double *d_db, double *d_dG, double *d_dA, int *d_status)
+{
+    if (const int rc = adjoint_check(bt, batch, d_Gs, d_As, d_x, d_y, d_z, d_s, d_exitflag))
+        return rc;
+    try
+    {
+        if (bt->eng->instance_matrices())
+            bt->eng->set_matrices(d_Gs, d_As, bt->rawG.data(), bt->rawA.data());
+        bt->eng->adjoint(batch, d_x, d_y, d_z, d_s, d_exitflag, d_gx, d_gy, d_gz, d_dc, d_dh, d_db, d_dG, d_dA, d_status);
+        return 0;
+    }
+    catch (const std::invalid_argument &e)
+    {
+        return fail(EICOS_ERR_INVALID, e.what());
+    }
+    catch (const std::exception &e)
+    {
+        return fail(EICOS_ERR_DEVICE, e.what());
+    }
+}
+
+int eicos_batch_adjoint(eicos_batch *bt, int batch, const double *Gs, const double *As,
+                        const double *x, const double *y, const double *z, const double *s, const int *exitflag,
+                        const double *gx, const double *gy, const double *gz,
+                        double *dc, double *dh, double *db, double *dG, double *dA, int *status)
+{
+    if (const int rc = adjoint_check(bt, batch, Gs, As, x, y, z, s, exitflag))
+        return rc;
+    try
+    {
+        const Symbolic &S = bt->S;
+        be::set_device(bt->device);
+        be::stream_t st = (be::stream_t)(intptr_t)bt->eng->stream();
+        // segments of at most `capacity` instances, as in eicos_batch_solve_matrices: staging bounded by the handle
+        const size_t cap = (size_t)std::max<long long>(1, bt->eng->capacity());
+        const size_t n = S.n, m = S.m, p = S.p, nG = S.G.nnz(), nA = S.A.nnz();
+        for (size_t first = 0; first < (size_t)batch; first += cap)
+        {
+            const size_t B = std::min(cap, (size_t)batch - first);
+            if (bt->eng->instance_matrices())
+            {
+                const size_t ng = Gs ? B * nG : 0, na = As ? B * nA : 0;
+                bt->dmat.ensure((ng + na) * sizeof(double));
+                double *dm = (double *)bt->dmat.p;
+                be::h2d(dm, Gs ? Gs + first * nG : nullptr, ng * sizeof(double), st);
+                be::h2d(dm + ng, As ? As + first * nA : nullptr, na * sizeof(double), st);
+                bt->eng->set_matrices(Gs ? dm : nullptr, As ? dm + ng : nullptr, bt->rawG.data(), bt->rawA.data());
+            }
+            // inputs: x, y, z, s, then the incoming gradients that are given
+            const size_t ix = B * n, iy = B * p, iz = B * m;
+            const size_t jx = gx ? ix : 0, jy = gy ? iy : 0, jz = gz ? iz : 0;
+            bt->din.ensure((ix + iy + 2 * iz + jx + jy + jz) * sizeof(double));
+            double *di = (double *)bt->din.p;
+            double *dx = di, *dy = dx + ix, *dz = dy + iy, *dsl = dz + iz, *dgx = dsl + iz, *dgy = dgx + jx, *dgz = dgy + jy;
+            be::h2d(dx, x ? x + first * n : nullptr, ix * sizeof(double), st);
+            be::h2d(dy, y ? y + first * p : nullptr, iy * sizeof(double), st);
+            be::h2d(dz, z ? z + first * m : nullptr, iz * sizeof(double), st);
+            be::h2d(dsl, s ? s + first * m : nullptr, iz * sizeof(double), st);
+            be::h2d(dgx, gx ? gx + first * n : nullptr, jx * sizeof(double), st);
+            be::h2d(dgy, gy ? gy + first * p : nullptr, jy * sizeof(double), st);
+            be::h2d(dgz, gz ? gz + first * m : nullptr, jz * sizeof(double), st);
+            // outputs that are wanted
+            const size_t oc = dc ? B * n : 0, oh = dh ? B * m : 0, ob = db ? B * p : 0, oG = dG ? B * nG : 0, oA = dA ? B * nA : 0;
+            bt->dout.ensure((oc + oh + ob + oG + oA) * sizeof(double));
+            double *dout = (double *)bt->dout.p;
+            double *odc = dout, *odh = odc + oc, *odb = odh + oh, *odG = odb + ob, *odA = odG + oG;
+            bt->dint.ensure(2 * B * sizeof(int));
+            int *dex = (int *)bt->dint.p, *dst = dex + B;
+            be::h2d(dex, exitflag + first, B * sizeof(int), st);
+            bt->eng->adjoint((int)B, dx, dy, dz, dsl, dex, gx ? dgx : nullptr, gy ? dgy : nullptr, gz ? dgz : nullptr,
+                             dc ? odc : nullptr, dh ? odh : nullptr, db ? odb : nullptr, dG ? odG : nullptr,
+                             dA ? odA : nullptr, dst);
+            be::d2h(dc ? dc + first * n : nullptr, odc, oc * sizeof(double), st);
+            be::d2h(dh ? dh + first * m : nullptr, odh, oh * sizeof(double), st);
+            be::d2h(db ? db + first * p : nullptr, odb, ob * sizeof(double), st);
+            be::d2h(dG ? dG + first * nG : nullptr, odG, oG * sizeof(double), st);
+            be::d2h(dA ? dA + first * nA : nullptr, odA, oA * sizeof(double), st);
+            be::d2h(status ? status + first : nullptr, dst, (status ? B : 0) * sizeof(int), st);
+            be::sync(st);
+        }
+        return 0;
+    }
+    catch (const std::invalid_argument &e)
+    {
+        return fail(EICOS_ERR_INVALID, e.what());
+    }
+    catch (const std::exception &e)
+    {
+        return fail(EICOS_ERR_DEVICE, e.what());
+    }
+}
+
 int eicos_batch_set_timing(eicos_batch *bt, int enabled)
 {
     if (!bt)

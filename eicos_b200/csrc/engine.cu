@@ -56,6 +56,25 @@ EI_DEFINE_KERNEL(eicos_debug_line_search, tile_debug_line_search, 2)
 #define EI_LAUNCH_JOBS(name, fn, tiles, njobs, threads, smem, stream, args) \
     name<<<(tiles) * (njobs), (threads), (smem), (stream)>>>(args)
 
+/* adjoint (Engine::adjoint): vector kernels with a second parameter block for the caller's pointers */
+#define EI_DEFINE_ADJ_KERNEL(name, fn)                                                                                   \
+    __global__ void __launch_bounds__(EI_MAX_THREADS, 2) name(const __grid_constant__ KArgs a, const __grid_constant__ AdjArgs g) \
+    {                                                                                                                      \
+        extern __shared__ double smem[];                                                                                   \
+        Team tm;                                                                                                           \
+        tm.pl = threadIdx.x & 31;                                                                                          \
+        tm.lane = tm.pl * VEC;                                                                                             \
+        tm.wk = threadIdx.x >> 5;                                                                                          \
+        tm.nwk = blockDim.x >> 5;                                                                                          \
+        tm.red = smem;                                                                                                     \
+        tm.pbuf = smem + (size_t)tm.nwk * KRED * TILE;                                                                     \
+        tm.job = 0;                                                                                                        \
+        fn(tm, a, g, (int)blockIdx.x);                                                                                     \
+    }
+EI_DEFINE_ADJ_KERNEL(eicos_adjoint_load, tile_adjoint_load)
+EI_DEFINE_ADJ_KERNEL(eicos_adjoint_store, tile_adjoint_store)
+#define EI_LAUNCH_ADJ(name, fn, tiles, threads, smem, stream, args, adj) name<<<(tiles), (threads), (smem), (stream)>>>(args, adj)
+
 __global__ void eicos_compact(const __grid_constant__ KArgs a, const __grid_constant__ MoveRanges mr, const int *moves)
 {
     const int src = moves[2 * blockIdx.x], dst = moves[2 * blockIdx.x + 1];
@@ -97,6 +116,15 @@ __global__ void eicos_compact(const __grid_constant__ KArgs a, const __grid_cons
             for (auto &t_ : th_)                                                                  \
                 t_.join();                                                                        \
         }                                                                                         \
+    } while (0)
+#endif
+
+#ifdef EICOS_EMU
+#define EI_LAUNCH_ADJ(name, fn, tiles, threads, smem, stream, args, adj)                                    \
+    do                                                                                                      \
+    {                                                                                                       \
+        const auto fn_ = [&](const Team &tm_, const KArgs &a_, int tile_) { fn(tm_, a_, (adj), tile_); }; \
+        EI_LAUNCH(name, fn_, tiles, threads, smem, stream, args);                                           \
     } while (0)
 #endif
 
@@ -259,12 +287,13 @@ void Engine::upload_pattern(const Symbolic &S)
     P.pim = pim_ ? 1 : 0;
     P.nnzG = S.G.nnz();
     P.nnzA = S.A.nnz();
+    // CSC index arrays of G and A: the on-device equilibration and the adjoint's per-entry gradients walk them
+    P.Gp = upload(S.G.p, owned_, st);
+    P.Gi = upload(S.G.i, owned_, st);
+    P.Ap = upload(S.A.p, owned_, st);
+    P.Ai = upload(S.A.i, owned_, st);
     if (pim_)
     {
-        P.Gp = upload(S.G.p, owned_, st);
-        P.Gi = upload(S.G.i, owned_, st);
-        P.Ap = upload(S.A.p, owned_, st);
-        P.Ai = upload(S.A.i, owned_, st);
         P.Grp = upload(S.Gr.p, owned_, st);
         P.Grv = upload(S.Gr.v, owned_, st);
         P.Arp = upload(S.Ar.p, owned_, st);
@@ -466,7 +495,7 @@ Engine::Engine(const Symbolic &S, int device, long long capacity_instances, int 
         const void *ks[] = {(const void *)eicos_load_inputs, (const void *)eicos_equilibrate, (const void *)eicos_init,
                             (const void *)eicos_init_point,
                             (const void *)eicos_iter_head, (const void *)eicos_iter_mid, (const void *)eicos_iter_tail,
-                            (const void *)eicos_store_outputs};
+                            (const void *)eicos_store_outputs, (const void *)eicos_adjoint_load, (const void *)eicos_adjoint_store};
         for (const void *k : ks)
             EI_CUDA(cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_common_));
     }
@@ -851,6 +880,78 @@ void Engine::solve(int batch, const double *d_c, const double *d_h, const double
     }
 #endif
 #undef EI_TIMED
+}
+
+void Engine::adjoint(int batch, const double *d_x, const double *d_y, const double *d_z, const double *d_s, const int *d_exit,
+                     const double *d_gx, const double *d_gy, const double *d_gz,
+                     double *d_dc, double *d_dh, double *d_db, double *d_dG, double *d_dA, int *d_status)
+{
+    be::set_device(device_);
+    be::stream_t st = S_(stream_);
+    if (batch <= 0)
+        return;
+    if ((!d_x && P_.n) || (!d_y && P_.p) || (!d_z && P_.m) || (!d_s && P_.m) || !d_exit)
+        throw std::invalid_argument("adjoint: x, y, z, s and the exit flags are required");
+    KArgs a;
+    std::memset(&a, 0, sizeof(a));
+    a.P = P_;
+    a.L = L_;
+    a.ws = ws_;
+    a.iws = iws_;
+    a.settings = settings_;
+    a.njobs = 1;
+    a.part_doubles = (int)part_doubles_;
+    if (pim_)
+    { // eicos_load_inputs brings this chunk's matrices (and vectors nobody reads here: zeros)
+        be::zero(base_vec_, (size_t)(P_.n + P_.m + P_.p) * sizeof(double), st);
+        a.base_c = base_vec_;
+        a.base_h = base_vec_ + P_.n;
+        a.base_b = base_vec_ + P_.n + P_.m;
+        a.in_G = mat_dG_;
+        a.in_A = mat_dA_;
+        a.base_G = base_mat_;
+        a.base_A = base_mat_ + nnzG_;
+    }
+    AdjArgs g;
+    g.x = d_x, g.y = d_y, g.z = d_z, g.s = d_s, g.exit = d_exit;
+    g.gx = d_gx, g.gy = d_gy, g.gz = d_gz;
+    g.dc = d_dc, g.dh = d_dh, g.db = d_db, g.dG = d_dG, g.dA = d_dA, g.status = d_status;
+    const int threads = workers_ * (LANES == 1 ? 1 : 32), threads1 = LANES == 1 ? 1 : 32;
+    const int threads_wide = M_MV_PARTS * (LANES == 1 ? 1 : 32);
+    (void)threads;
+    (void)threads1;
+    (void)threads_wide;
+    for (long long first = 0; first < batch; first += cap_tiles_ * TILE)
+    {
+        const int nb = (int)std::min<long long>(batch - first, cap_tiles_ * TILE);
+        const int tiles = (nb + TILE - 1) / TILE;
+        a.batch = nb;
+        a.first = (int)first;
+        if (pim_)
+        {
+            EI_LAUNCH(eicos_load_inputs, tile_load, tiles, threads, smem_common_, st, a);
+            EI_LAUNCH(eicos_equilibrate, tile_equil, tiles, threads, smem_common_, st, a);
+        }
+        EI_LAUNCH_ADJ(eicos_adjoint_load, tile_adjoint_load, tiles, threads, smem_common_, st, a, g);
+        a.variant = deep_ring(tiles) ? M_VARIANTS - 1 : 0;
+        EI_LAUNCH(eicos_ldl_factor, tile_factor, tiles, threads1, smem_factor_[a.variant], st, a);
+        // one solveKKT (rhs1 -> sol1) in the form and ring depth a one-job solve of the iteration takes
+        a.job[0] = {L_.rhs1, L_.sol1, J_NIT1, 0};
+        a.initialize = 0;
+        a.variant = deep_ring(tiles) ? M_VARIANTS - 1 : 0;
+        if (wide_launch(tiles))
+        {
+            a.variant = force_variant_ == 0 ? 0 : M_VARIANTS - 1;
+            EI_LAUNCH_JOBS(eicos_solve_kkt_wide, tile_solve_kkt<1>, tiles, 1, threads_wide, smem_wide_, st, a);
+        }
+        else
+            EI_LAUNCH_JOBS(eicos_solve_kkt, tile_solve_kkt<1>, tiles, 1, threads1, smem_prog_[a.variant], st, a);
+        EI_LAUNCH_ADJ(eicos_adjoint_store, tile_adjoint_store, tiles, threads, smem_common_, st, a, g);
+    }
+#ifndef EICOS_EMU
+    EI_CUDA(cudaGetLastError());
+#endif
+    be::sync(st);
 }
 
 void Engine::debug_factor_init(int batch, const double *d_c, const double *d_h, const double *d_b,

@@ -83,6 +83,15 @@ class Engine
                int *d_exit, int *d_iter, double *d_info, int *d_iinfo,
                bool keep_sticky, bool pre_equilibrated, bool timing, SolveStats *stats);
 
+    // Gradients of the solution map for `batch` instances (no state kept from the solve): one factorisation of the
+    // KKT matrix at the given (s, z) and one solveKKT per instance.  d_x .. d_exit: the forward's results, d_gx / d_gy /
+    // d_gz: incoming gradients (null = zero); outputs dc [batch x n], dh [batch x m], db [batch x p], dG [batch x nnzG],
+    // dA [batch x nnzA], status [batch] (any may be null).  All instance-major DEVICE arrays, original scaling, z-shaped
+    // arrays in compact z order.  Per-instance-matrices handles use the matrices of set_matrices().  Blocks until done.
+    void adjoint(int batch, const double *d_x, const double *d_y, const double *d_z, const double *d_s, const int *d_exit,
+                 const double *d_gx, const double *d_gy, const double *d_gz,
+                 double *d_dc, double *d_dh, double *d_db, double *d_dG, double *d_dA, int *d_status);
+
     // debug entry points (GPU unit tests): run the initial factorisation / one KKT solve for
     // instance-major data and copy raw factor values back (host pointers, may be null)
     void debug_factor_init(int batch, const double *d_c, const double *d_h, const double *d_b,

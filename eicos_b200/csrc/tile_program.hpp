@@ -1730,6 +1730,51 @@ EI_DEV ConeScaling cone_scaling(const Team &tm, const double *T, int srow, int z
     return r;
 }
 
+// the scaling rows of cone c (cpar block cp, q rows from qo) for one instance from cone_scaling() of (srow, zrow):
+// eta and q for stage 0 and 2, the rest for stage 0 only (updateScalings, src/eicos.cpp:419-474)
+EI_DEV void cone_scaling_rows(double *T, const Layout &L, int cp, int qo, int srow, int zrow, int d, const ConeScaling &cs, int c)
+{
+    ROWC(T, cp + CP_ETA2, c) = cs.eta2;
+    ROWC(T, cp + CP_ETA, c) = cs.eta;
+    for (int k = 1; k < d; k++)
+        ROWC(T, L.cq + qo + k - 1, c) = (0.5 / cs.gamma) * (ROWC(T, srow + k, c) / cs.snorm - ROWC(T, zrow + k, c) / cs.znorm);
+    if (cs.stage == 2)
+        return;
+    ROWC(T, cp + CP_D1, c) = cs.d1;
+    ROWC(T, cp + CP_U0, c) = cs.u0;
+    ROWC(T, cp + CP_U1, c) = cs.u1;
+    ROWC(T, cp + CP_V1, c) = cs.v1;
+    ROWC(T, cp + CP_A, c) = cs.a;
+    ROWC(T, cp + CP_W, c) = cs.w;
+}
+
+// updateKKTScalings (src/eicos.cpp:1691-1732), second-order cone part: the V rows of every cone from its scaling rows
+EI_DEV void cone_kkt_scalings(const Team &tm, const KArgs &a, double *T)
+{
+    const DevPattern &P = a.P;
+    const Layout &L = a.L;
+    const double delta = Settings::deltastat;
+    for (int c = tm.wk; c < P.nc; c += tm.nwk)
+    {
+        const int d = EI_LDG(P.cone_dim + c), ks = EI_LDG(P.cone_k + c), qo = EI_LDG(P.cone_q + c);
+        const int cp = L.cpar + c * CP_COUNT;
+        const vd eta2 = ROWD(T, cp + CP_ETA2), d1 = ROWD(T, cp + CP_D1), u0 = ROWD(T, cp + CP_U0);
+        const vd u1 = ROWD(T, cp + CP_U1), v1 = ROWD(T, cp + CP_V1);
+        // cones before c contributed sum(3 dim + 1) V entries; ks - 2c - l = sum of their dims
+        int vb_ = L.V + P.l + 3 * (ks - 2 * c - P.l) + c;
+        ROWD(T, vb_++) = -(eta2 * d1) - delta;
+        for (int k = 1; k < d; k++)
+            ROWD(T, vb_++) = -eta2 - delta;
+        ROWD(T, vb_++) = -eta2;
+        for (int k = 1; k < d; k++)
+            ROWD(T, vb_++) = -(eta2 * v1) * vd(ROWD(T, L.cq + qo + k - 1));
+        ROWD(T, vb_++) = eta2 + delta;
+        ROWD(T, vb_++) = -(eta2 * u0);
+        for (int k = 1; k < d; k++)
+            ROWD(T, vb_++) = -(eta2 * u1) * vd(ROWD(T, L.cq + qo + k - 1));
+    }
+}
+
 // ------------------------------------------------------------------ computeResiduals (src/eicos.cpp:643-689)
 // rx = -A'y - G'z, ry = A x, rz = s + G x (each before and after the tau terms) and the sums the
 // statistics need; one warp per tile runs the machine program of streams.cpp: build_resid, whose
@@ -2104,18 +2149,7 @@ EI_DEV void tile_head(const Team &tm, const KArgs &a, int tile)
                 const ConeScaling cs = cone_scaling(tm, T, L.s + ks, sz + ks, d, c_);
                 if (cs.stage == 1)
                     continue;
-                ROWC(T, cp + CP_ETA2, c_) = cs.eta2;
-                ROWC(T, cp + CP_ETA, c_) = cs.eta;
-                for (int k = 1; k < d; k++)
-                    ROWC(T, L.cq + qo + k - 1, c_) = (0.5 / cs.gamma) * (ROWC(T, L.s + ks + k, c_) / cs.snorm - ROWC(T, sz + ks + k, c_) / cs.znorm);
-                if (cs.stage == 2)
-                    continue;
-                ROWC(T, cp + CP_D1, c_) = cs.d1;
-                ROWC(T, cp + CP_U0, c_) = cs.u0;
-                ROWC(T, cp + CP_U1, c_) = cs.u1;
-                ROWC(T, cp + CP_V1, c_) = cs.v1;
-                ROWC(T, cp + CP_A, c_) = cs.a;
-                ROWC(T, cp + CP_W, c_) = cs.w;
+                cone_scaling_rows(T, L, cp, qo, L.s + ks, sz + ks, d, cs, c_);
             }
         }
     }
@@ -2124,26 +2158,7 @@ EI_DEV void tile_head(const Team &tm, const KArgs &a, int tile)
         cone_scale(tm, a, T, sz, L.lam, cont && nofail);
 
     // ---- updateKKTScalings (:1691-1732) into the V rows, RHSaffine (:1670-1689) into rhs2
-    const double delta = Settings::deltastat;
-    for (int c = tm.wk; c < P.nc; c += tm.nwk)
-    {
-        const int d = EI_LDG(P.cone_dim + c), ks = EI_LDG(P.cone_k + c), qo = EI_LDG(P.cone_q + c);
-        const int cp = L.cpar + c * CP_COUNT;
-        const vd eta2 = ROWD(T, cp + CP_ETA2), d1 = ROWD(T, cp + CP_D1), u0 = ROWD(T, cp + CP_U0);
-        const vd u1 = ROWD(T, cp + CP_U1), v1 = ROWD(T, cp + CP_V1);
-        // cones before c contributed sum(3 dim + 1) V entries; ks - 2c - l = sum of their dims
-        int vb_ = L.V + P.l + 3 * (ks - 2 * c - P.l) + c;
-        ROWD(T, vb_++) = -(eta2 * d1) - delta;
-        for (int k = 1; k < d; k++)
-            ROWD(T, vb_++) = -eta2 - delta;
-        ROWD(T, vb_++) = -eta2;
-        for (int k = 1; k < d; k++)
-            ROWD(T, vb_++) = -(eta2 * v1) * vd(ROWD(T, L.cq + qo + k - 1));
-        ROWD(T, vb_++) = eta2 + delta;
-        ROWD(T, vb_++) = -(eta2 * u0);
-        for (int k = 1; k < d; k++)
-            ROWD(T, vb_++) = -(eta2 * u1) * vd(ROWD(T, L.cq + qo + k - 1));
-    }
+    cone_kkt_scalings(tm, a, T);
     {
         vd mx[1] = {vset(0.0)}; // max |rhs2| for the affine solve
         const int ins[1] = {L.r};
@@ -2714,6 +2729,227 @@ EI_DEV void compact_vacate(const KArgs &a, int src)
     SI[(size_t)J_STATUS * TILE] = EXIT_FATAL;
     SI[(size_t)J_INST * TILE] = -1;
     SI[(size_t)J_STORED * TILE] = 1;
+}
+
+// ------------------------------------------------------------------ adjoint of the solution map (Engine::adjoint)
+// Pointers of one adjoint call: the forward's results and the incoming gradients in, the gradients with respect to
+// the problem data out; instance-major, original (unequilibrated) scaling, z-shaped arrays in compact z order.
+// gx / gy / gz null: zero; any output may be null.
+struct AdjArgs
+{
+    const double *x, *y, *z, *s;
+    const int *exit;
+    const double *gx, *gy, *gz;
+    double *dc, *dh, *db, *dG, *dA;
+    int *status;
+};
+
+// per-instance status of an adjoint (include/eicos_b200.h)
+enum : int
+{
+    ADJ_OK = 0,
+    ADJ_NOT_OPTIMAL = 1,  // exit flag other than 0 / 10
+    ADJ_NOT_INTERIOR = 2, // an LP s or z <= 0, or a cone's s or z not strictly inside
+    ADJ_NOT_FINITE = 3    // the KKT solve gave a non-finite value
+};
+
+// equilibration scale of KKT row q for this lane's instances: [x_equil | A_equil | G_equil expanded] (1 in the slots)
+EI_DEV vd adj_eq(const KArgs &a, const double *T, int q)
+{
+    if (a.P.pim)
+        return vload(T + (size_t)(a.L.eq + q) * TILE);
+    const int n = a.P.n, zb = a.P.n + a.P.p;
+    return vset(q < n ? EI_LDG(a.P.xeq + q) : (q < zb ? EI_LDG(a.P.Aeq + q - n) : EI_LDG(a.P.GeqE + q - zb)));
+}
+
+// Loads the iterate and the incoming gradients of the chunk's instances, builds the Nesterov-Todd scalings of the
+// equilibrated (s, z) into the scaling rows and the V block (what the head step's updateScalings / updateKKTScalings
+// write), and rhs1 = D^-1 [gx; gy; gz] with D = diag(x_equil, A_equil, G_equil).  The lanes to differentiate are
+// left ST_ACTIVE, so that the factorisation and solveKKT run on them only; every other lane is frozen with its
+// ADJ_* status.  Rows: w = [x | y | z] (original scaling), s = s_e = s / G_equil, lam = z_e = z * G_equil.
+EI_DEV void tile_adjoint_load(const Team &tm, const KArgs &a, const AdjArgs &g, int tile)
+{
+    const TileMem t = tile_mem(tm, a, tile);
+    const DevPattern &P = a.P;
+    const Layout &L = a.L;
+    double *T = t.T;
+    const int n = P.n, zb = P.n + P.p;
+    bool valid[VEC];
+    size_t gi[VEC];
+    VFOR
+    {
+        int inst = tile * TILE + tm.lane + c_;
+        valid[c_] = inst < a.batch;
+        if (!valid[c_])
+            inst = a.batch - 1; // padding lanes replay the last instance; nothing of theirs is stored
+        gi[c_] = (size_t)a.first + inst;
+    }
+    vd red[2] = {vset(0.0), vset(0.0)}; // max |rhs1|, "not interior"
+    for (int j = tm.wk; j < n; j += tm.nwk)
+    {
+        vd xv, gv;
+        VFOR
+        {
+            xv.v[c_] = g.x[gi[c_] * n + j];
+            gv.v[c_] = g.gx ? g.gx[gi[c_] * n + j] : 0.0;
+        }
+        const vd r = gv / adj_eq(a, T, j);
+        ROWD(T, L.w + j) = xv;
+        ROWD(T, L.rhs1 + j) = r;
+        red[0] = vmax(red[0], vabs(r));
+    }
+    for (int i = tm.wk; i < P.p; i += tm.nwk)
+    {
+        vd yv, gv;
+        VFOR
+        {
+            yv.v[c_] = g.y[gi[c_] * P.p + i];
+            gv.v[c_] = g.gy ? g.gy[gi[c_] * P.p + i] : 0.0;
+        }
+        const vd r = gv / adj_eq(a, T, n + i);
+        ROWD(T, L.w + n + i) = yv;
+        ROWD(T, L.rhs1 + n + i) = r;
+        red[0] = vmax(red[0], vabs(r));
+    }
+    for (int i = tm.wk; i < P.m; i += tm.nwk)
+    {
+        const int e = EI_LDG(P.zk + i);
+        vd zv, sv, gv;
+        VFOR
+        {
+            zv.v[c_] = g.z[gi[c_] * P.m + i];
+            sv.v[c_] = g.s[gi[c_] * P.m + i];
+            gv.v[c_] = g.gz ? g.gz[gi[c_] * P.m + i] : 0.0;
+        }
+        const vd eq = adj_eq(a, T, zb + e), r = gv / eq;
+        ROWD(T, L.w + zb + e) = zv;
+        ROWD(T, L.s + e) = sv / eq;
+        ROWD(T, L.lam + e) = zv * eq;
+        ROWD(T, L.rhs1 + zb + e) = r;
+        red[0] = vmax(red[0], vabs(r));
+    }
+    for (int c = tm.wk; c < P.nc; c += tm.nwk)
+    { // the two expansion slots of every cone: zero in every z-shaped row
+        const int e = EI_LDG(P.cone_k + c) + EI_LDG(P.cone_dim + c);
+        for (int k = e; k < e + 2; k++)
+        {
+            ROWD(T, L.w + zb + k) = 0.0;
+            ROWD(T, L.s + k) = 0.0;
+            ROWD(T, L.lam + k) = 0.0;
+            ROWD(T, L.rhs1 + zb + k) = 0.0;
+        }
+    }
+    tm.sync(); // the rows above are complete before the passes below, which split them differently
+    // updateScalings (src/eicos.cpp:411-479) of (s_e, z_e) and updateKKTScalings (:1691-1732)
+    for (int k = tm.wk; k < P.l; k += tm.nwk)
+    {
+        const vd sv = ROWD(T, L.s + k), zv = ROWD(T, L.lam + k);
+        const vd v = sv / zv;
+        ROWD(T, L.lpv + k) = -v;
+        ROWD(T, L.lpw + k) = vsqrt(v);
+        ROWD(T, L.V + k) = -v - Settings::deltastat;
+        VFOR if (!(sv.v[c_] > 0 && zv.v[c_] > 0)) red[1].v[c_] = 1.0;
+    }
+    for (int c = tm.wk; c < P.nc; c += tm.nwk)
+    {
+        const int d = EI_LDG(P.cone_dim + c), ks = EI_LDG(P.cone_k + c), qo = EI_LDG(P.cone_q + c);
+        VFOR
+        {
+            const ConeScaling cs = cone_scaling(tm, T, L.s + ks, L.lam + ks, d, c_);
+            if (cs.stage != 0)
+                red[1].v[c_] = 1.0;
+            else
+                cone_scaling_rows(T, L, L.cpar + c * CP_COUNT, qo, L.s + ks, L.lam + ks, d, cs, c_);
+        }
+    }
+    team_max<2>(tm, red);
+    cone_kkt_scalings(tm, a, T); // (cone c's scaling rows were written by this worker)
+    if (tm.wk == 0)
+        VFOR
+        {
+            const int ex = g.exit[gi[c_]];
+            const int st = ex != EXIT_OPTIMAL && ex != EXIT_OPTIMAL + EXIT_INACC ? ADJ_NOT_OPTIMAL
+                           : red[1].v[c_] != 0.0                               ? ADJ_NOT_INTERIOR
+                                                                               : (int)ST_ACTIVE;
+            ROWC(t.I, J_STATUS, c_) = valid[c_] ? st : (int)EXIT_FATAL;
+            ROWC(t.I, J_INST, c_) = valid[c_] ? (int)gi[c_] : -1;
+            ROWC(T, L.sc + S_RHSMAX1, c_) = red[0].v[c_];
+        }
+}
+
+// After the factorisation and solveKKT (rhs1 -> sol1): u = D^-1 sol1 solves K0 u = g in the original scaling.
+// Writes dc = -u_x, db = u_y, dh = u_z, and per pattern entry dG_ij = -(z_i u_x,j + u_z,i x_j),
+// dA_ij = -(y_i u_x,j + u_y,i x_j) (CSC order), and the status of every instance.  The outer products run down the
+// rows (one 16-byte access per lane and row) and are written instance-major; lanes not differentiated get zeros.
+EI_DEV void tile_adjoint_store(const Team &tm, const KArgs &a, const AdjArgs &g, int tile)
+{
+    const TileMem t = tile_mem(tm, a, tile);
+    const DevPattern &P = a.P;
+    const Layout &L = a.L;
+    double *T = t.T;
+    const int n = P.n, zb = P.n + P.p;
+    vb diff;
+    VFOR diff.v[c_] = ROWC(t.I, J_STATUS, c_) == ST_ACTIVE;
+    vd bad[1] = {vset(0.0)};
+    for (int q = tm.wk; q < P.N; q += tm.nwk)
+    {
+        const vd u = vd(ROWD(T, L.sol1 + q)) / adj_eq(a, T, q);
+        ROWD(T, L.sol1 + q) = u;
+        VFOR if (!(fabs(u.v[c_]) <= DBL_MAX)) bad[0].v[c_] = 1.0;
+    }
+    team_max<1>(tm, bad); // (its barriers also complete u before the passes below)
+    int code[VEC];
+    VFOR
+    {
+        const int st = ROWC(t.I, J_STATUS, c_);
+        code[c_] = st == ST_ACTIVE ? (bad[0].v[c_] != 0.0 ? ADJ_NOT_FINITE : ADJ_OK) : (st == EXIT_FATAL ? ADJ_NOT_FINITE : st);
+        diff.v[c_] = diff.v[c_] && code[c_] == ADJ_OK;
+    }
+    const vd zero = vset(0.0);
+    const auto put = [&](double *out, int stride, int k, vd v) {
+        v = vsel(diff, v, zero);
+        VFOR
+        {
+            const int inst = ROWC(t.I, J_INST, c_);
+            if (inst >= 0)
+                out[(size_t)inst * stride + k] = v.v[c_];
+        }
+    };
+    if (g.dc)
+        for (int j = tm.wk; j < n; j += tm.nwk)
+            put(g.dc, n, j, -vd(ROWD(T, L.sol1 + j)));
+    if (g.db)
+        for (int i = tm.wk; i < P.p; i += tm.nwk)
+            put(g.db, P.p, i, ROWD(T, L.sol1 + n + i));
+    if (g.dh)
+        for (int i = tm.wk; i < P.m; i += tm.nwk)
+            put(g.dh, P.m, i, ROWD(T, L.sol1 + zb + EI_LDG(P.zk + i)));
+    // (a problem without G or A may come without its column pointers)
+    const bool wG = g.dG && P.nnzG > 0, wA = g.dA && P.nnzA > 0;
+    if (wG || wA)
+        for (int j = tm.wk; j < n; j += tm.nwk)
+        {
+            const vd xj = ROWD(T, L.w + j), uxj = ROWD(T, L.sol1 + j);
+            if (wG)
+                for (int k = EI_LDG(P.Gp + j), k1 = EI_LDG(P.Gp + j + 1); k < k1; k++)
+                {
+                    const int r = zb + EI_LDG(P.zk + EI_LDG(P.Gi + k));
+                    put(g.dG, P.nnzG, k, -(vd(ROWD(T, L.w + r)) * uxj + vd(ROWD(T, L.sol1 + r)) * xj));
+                }
+            if (wA)
+                for (int k = EI_LDG(P.Ap + j), k1 = EI_LDG(P.Ap + j + 1); k < k1; k++)
+                {
+                    const int r = n + EI_LDG(P.Ai + k);
+                    put(g.dA, P.nnzA, k, -(vd(ROWD(T, L.w + r)) * uxj + vd(ROWD(T, L.sol1 + r)) * xj));
+                }
+        }
+    if (tm.wk == 0 && g.status)
+        VFOR
+        {
+            const int inst = ROWC(t.I, J_INST, c_);
+            if (inst >= 0)
+                g.status[inst] = code[c_];
+        }
 }
 
 } // namespace eicos

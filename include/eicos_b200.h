@@ -165,6 +165,43 @@ int eicos_batch_solve_matrices_device(eicos_batch *bt, int batch, const double *
                                       double *d_x, double *d_y, double *d_z, double *d_s,
                                       int *d_exitflag, int *d_iters);
 
+/* ---- gradients of the solution map (the backward pass of a batched solve)
+ * Problem: min c'x  s.t.  A x = b,  G x + s = h,  s in K.  At a solution (x, y, z, s) of eicos_batch_solve*, with the
+ * complementarity linearised by the Nesterov-Todd scaling W of (s, z) as in the solver's Newton steps
+ * (ds = -W'W dz; LP rows: W^2 = s / z), the derivative of (x, y, z) satisfies
+ *     K0 [dx; dy; dz] = [-dc - dA'y - dG'z;  db - dA x;  dh - dG x],   K0 = [0 A' G'; A 0 0; G 0 -W^2].
+ * Given the gradients gx, gy, gz of a loss with respect to x, y, z, one solve K0 u = [gx; gy; gz] per instance
+ * (the factorisation and the refined solve of the solver's Newton steps, on the equilibrated system) gives
+ *     dL/dc = -u_x,  dL/db = u_y,  dL/dh = u_z,
+ *     dL/dA_ij = -(y_i u_x,j + u_y,i x_j),  dL/dG_ij = -(z_i u_x,j + u_z,i x_j)   (on the pattern, CSC order).
+ * This is the exact derivative of the central-path point at the final iterate's mu; it tends to the derivative of
+ * the solution as mu -> 0 where complementarity is strict.  Like every Newton step of the solver the solve carries
+ * the static regularisation (7e-8 on the diagonal), so u solves K0 u = g up to about 7e-8 |u|.
+ *
+ * Arguments (instance-major, original scaling, z-shaped arrays in compact z order):
+ *   x [batch x n], y [batch x p], z, s [batch x m], exitflag [batch]: the forward's results (required);
+ *   gx, gy, gz: incoming gradients, NULL = zero;
+ *   dc [batch x n], dh [batch x m], db [batch x p], dG [batch x nnzG], dA [batch x nnzA], status [batch]:
+ *   outputs, any may be NULL;
+ *   Gs [batch x nnzG], As [batch x nnzA]: the forward's per-instance matrices on a handle from
+ *   eicos_batch_setup_ex(..., EICOS_BATCH_INSTANCE_MATRICES) (NULL = the setup values, as in a solve); they must be
+ *   NULL on a shared-matrices handle.
+ * The handle's current matrices (after eicos_batch_update_matrices) and settings (nitref, linsysacc, irerrfact) apply.
+ * Per-instance status: 0 differentiated; 1 exit flag other than 0 or 10; 2 not interior (an LP s or z <= 0, or a
+ * cone's s or z not strictly inside it); 3 the solve gave a non-finite value.  Instances with status != 0 get exact
+ * zeros in every output.  Returns EICOS_ERR_INVALID for batch <= 0, a missing required buffer or Gs / As given to a
+ * shared-matrices handle.  Nothing is kept between the forward and this call. */
+int eicos_batch_adjoint(eicos_batch *bt, int batch, const double *Gs, const double *As,
+                        const double *x, const double *y, const double *z, const double *s, const int *exitflag,
+                        const double *gx, const double *gy, const double *gz,
+                        double *dc, double *dh, double *db, double *dG, double *dA, int *status);
+/* The same with DEVICE buffers (results stay in HBM).  Runs on the engine's stream (eicos_batch_stream) and returns
+ * after it has drained. */
+int eicos_batch_adjoint_device(eicos_batch *bt, int batch, const double *d_Gs, const double *d_As,
+                               const double *d_x, const double *d_y, const double *d_z, const double *d_s,
+                               const int *d_exitflag, const double *d_gx, const double *d_gy, const double *d_gz,
+                               double *d_dc, double *d_dh, double *d_db, double *d_dG, double *d_dA, int *d_status);
+
 typedef struct eicos_batch_stats
 {
     int chunks, ipm_iterations;
