@@ -1,13 +1,23 @@
-"""PyTorch autograd layer over a batched solve and its adjoint (eicos_batch_solve*_device / eicos_batch_adjoint_device).
+"""PyTorch autograd layer over a batched solve, its adjoint and its tangent (eicos_batch_solve*_device,
+eicos_batch_adjoint_device, eicos_batch_tangent_device).
 
     layer = EiCOSLayer(BatchSolver(problem))
     x, y, z, exitflag = layer(c=cs, h=hs, b=bs)      # float64 tensors [batch, k]
     loss(x, y, z).backward()                          # cs.grad, hs.grad, bs.grad
 
+Forward mode (torch.autograd.forward_ad) runs the tangent: one call per direction, for every instance at once.
+
+    with fwAD.dual_level():
+        x, y, z, _ = layer(h=fwAD.make_dual(hs, dh))
+        dx = fwAD.unpack_dual(x).tangent                # derivative of x along dh
+
+Inputs that are not dual contribute nothing and are never read as tangents.  torch.func.jvp is not supported: it
+passes tensors without storage to forward(), and the library needs the tensors' memory.
+
 Inputs left as None use the handle's setup data and get no gradient; G / A (per-instance matrix values in CSC order)
 need a handle made with instance_matrices=True.  The forward keeps (x, y, z, s, exitflag) for the backward pass; s is
 not returned.  Instances whose adjoint status is not 0 (not optimal, not interior, not finite; include/eicos_b200.h)
-get zero gradients.
+get zero gradients (and zero tangents).
 
 The library reads and writes the tensors' memory directly: CUDA tensors with the CUDA library, CPU tensors with a
 library built for the host.  Before each call the engine's stream waits for the caller's current stream, so work
@@ -73,8 +83,26 @@ class _SolveFn(torch.autograd.Function):
         ctx.layer, ctx.batch, ctx.device = layer, batch, device
         ctx.given = tuple(data[k] is not None for k in _NAMES)
         ctx.save_for_backward(x, y, z, s, ex, data["G"], data["A"])
+        ctx.save_for_forward(x, y, z, s, ex, data["G"], data["A"])
+        # tangents of inputs that are not dual arrive as None (NULL: a G / A stack of zeros is never read); gradients
+        # that were not computed also arrive as None, which the adjoint takes as zero
+        ctx.set_materialize_grads(False)
         ctx.mark_non_differentiable(ex)
         return x, y, z, ex
+
+    @staticmethod
+    def jvp(ctx, _dlayer, dc, dh, db, dG, dA):
+        x, y, z, s, ex, G, A = ctx.saved_tensors
+        layer, batch, device = ctx.layer, ctx.batch, ctx.device
+        bs = layer.solver
+        v = [None if t is None else t.contiguous() for t in (dc, dh, db, dG, dA)]
+        f64 = dict(dtype=torch.float64, device=device)
+        dx, dy, dz = torch.empty(batch, bs.n, **f64), torch.empty(batch, bs.p, **f64), torch.empty(batch, bs.m, **f64)
+        layer._wait(device)
+        bs.tangent_device(batch, d_x=_ptr(x), d_y=_ptr(y), d_z=_ptr(z), d_s=_ptr(s), d_exit=_ptr(ex),
+                          d_dc=_ptr(v[0]), d_dh=_ptr(v[1]), d_db=_ptr(v[2]), d_dG=_ptr(v[3]), d_dA=_ptr(v[4]),
+                          d_ox=_ptr(dx), d_oy=_ptr(dy), d_oz=_ptr(dz), d_Gs=_ptr(G), d_As=_ptr(A))
+        return dx, dy, dz, None
 
     @staticmethod
     def backward(ctx, gx, gy, gz, _gex):

@@ -111,7 +111,7 @@ EXPORTS = [
     "eicos_batch_set_settings", "eicos_batch_get_settings", "eicos_multi_set_settings", "eicos_multi_get_settings",
     "eicos_batch_setup", "eicos_batch_setup_ex", "eicos_batch_update_matrices", "eicos_batch_solve",
     "eicos_batch_solve_matrices", "eicos_batch_solve_device", "eicos_batch_solve_matrices_device",
-    "eicos_batch_adjoint", "eicos_batch_adjoint_device",
+    "eicos_batch_adjoint", "eicos_batch_adjoint_device", "eicos_batch_tangent", "eicos_batch_tangent_device",
     "eicos_batch_set_timing", "eicos_batch_set_compaction", "eicos_batch_get_stats", "eicos_batch_get_dims", "eicos_batch_get_program_stats", "eicos_batch_get_symbolic",
     "eicos_batch_debug_init", "eicos_batch_debug_line_search", "eicos_batch_debug_set_iter_max", "eicos_batch_stream", "eicos_batch_cleanup",
     "eicos_multi_setup", "eicos_multi_solve", "eicos_multi_ngpu", "eicos_multi_slice", "eicos_multi_cleanup",
@@ -176,6 +176,10 @@ class Library:
         L.eicos_batch_adjoint.argtypes = [C.c_void_p, C.c_int] + [_dp] * 6 + [_ip] + [_dp] * 8 + [_ip]
         L.eicos_batch_adjoint_device.restype = C.c_int
         L.eicos_batch_adjoint_device.argtypes = [C.c_void_p, C.c_int] + [C.c_void_p] * 16
+        L.eicos_batch_tangent.restype = C.c_int
+        L.eicos_batch_tangent.argtypes = [C.c_void_p, C.c_int] + [_dp] * 6 + [_ip] + [_dp] * 9 + [_ip]
+        L.eicos_batch_tangent_device.restype = C.c_int
+        L.eicos_batch_tangent_device.argtypes = [C.c_void_p, C.c_int] + [C.c_void_p] * 17
         L.eicos_batch_set_timing.restype = C.c_int
         L.eicos_batch_set_timing.argtypes = [C.c_void_p, C.c_int]
         L.eicos_batch_set_compaction.restype = C.c_int
@@ -445,6 +449,53 @@ class BatchSolver(_HasSettings):
             self.h, int(batch), *[C.c_void_p(int(v) or None) for v in
                                   (d_Gs, d_As, d_x, d_y, d_z, d_s, d_exit, d_gx, d_gy, d_gz,
                                    d_dc, d_dh, d_db, d_dG, d_dA, d_status)]))
+
+    TANGENT_OUTPUTS = ("x", "y", "z", "s")
+
+    def tangent(self, out, dc=None, dh=None, db=None, dG=None, dA=None, Gs=None, As=None, want=TANGENT_OUTPUTS):
+        """Derivatives of the solutions `out` = solve(...) returned along a direction in the problem data
+        (eicos_batch_tangent): dc [batch x n], dh [batch x m], db [batch x p], dG [batch x nnzG], dA [batch x nnzA]
+        (CSC order; both kinds of handle); None = zero.  Gs / As: the forward's per-instance matrices
+        (instance-matrices handles only; None = the setup values).
+        Returns {"x": [batch x n], "y": [batch x p], "z": [batch x m], "s": [batch x m]} for the names in `want`, and
+        "status" [batch] (0 differentiated, 1 not optimal, 2 not interior, 3 not finite; instances with status != 0
+        get zeros)."""
+        unknown = sorted(set(want) - set(self.TANGENT_OUTPUTS))
+        if unknown:
+            raise ValueError(f"unknown tangent outputs: {', '.join(unknown)}")
+        batch = int(np.asarray(out["exit"]).size)
+        sizes = {"x": self.n, "y": self.p, "z": self.m, "s": self.m}
+        it = {k: np.ascontiguousarray(out[k], np.float64) for k in sizes}
+        ex = np.ascontiguousarray(out["exit"], np.int32)
+        dims = {"c": self.n, "h": self.m, "b": self.p, "G": self.nnzG, "A": self.nnzA}
+        v = {k: _arr(a, np.float64) for k, a in (("c", dc), ("h", dh), ("b", db), ("G", dG), ("A", dA))}
+        Gs, As = _arr(Gs, np.float64), _arr(As, np.float64)
+        for k, a in it.items():
+            if a.size != batch * sizes[k]:
+                raise ValueError(f"out[{k!r}] has the wrong size")
+        for k, a in v.items():
+            if a is not None and a.size != batch * dims[k]:
+                raise ValueError(f"d{k} has the wrong size")
+        for a, k in ((Gs, self.nnzG), (As, self.nnzA)):
+            if a is not None and a.size != batch * k:
+                raise ValueError("stacked matrix values have the wrong size")
+        res = {k: np.zeros((batch, sizes[k])) if k in want else None for k in self.TANGENT_OUTPUTS}
+        status = np.zeros(batch, np.int32)
+        self.lib.check(self.lib.L.eicos_batch_tangent(
+            self.h, batch, _d(Gs), _d(As), *[_d(it[k]) for k in "xyzs"], _i(ex),
+            *[_d(v[k]) for k in ("c", "h", "b", "G", "A")], *[_d(res[k]) for k in self.TANGENT_OUTPUTS], _i(status)))
+        res = {k: a for k, a in res.items() if a is not None}
+        res["status"] = status
+        return res
+
+    def tangent_device(self, batch, d_x=0, d_y=0, d_z=0, d_s=0, d_exit=0, d_dc=0, d_dh=0, d_db=0, d_dG=0, d_dA=0,
+                       d_ox=0, d_oy=0, d_oz=0, d_os=0, d_status=0, d_Gs=0, d_As=0):
+        """eicos_batch_tangent_device on raw device pointers (ints, 0 = NULL); results (d_ox .. d_os = dx, dy, dz,
+        ds) stay in HBM."""
+        self.lib.check(self.lib.L.eicos_batch_tangent_device(
+            self.h, int(batch), *[C.c_void_p(int(v) or None) for v in
+                                  (d_Gs, d_As, d_x, d_y, d_z, d_s, d_exit, d_dc, d_dh, d_db, d_dG, d_dA,
+                                   d_ox, d_oy, d_oz, d_os, d_status)]))
 
     def debug_line_search(self, lam, ds, dz, scalars):
         """lineSearch on caller data: lam, ds, dz [batch x m] in z order, scalars [batch x 4] = tau, dtau, kap, dkap."""

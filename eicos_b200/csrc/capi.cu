@@ -400,15 +400,15 @@ int eicos_batch_solve_matrices(eicos_batch *bt, int batch, const double *Gs, con
 }
 
 static int adjoint_check(const eicos_batch *bt, int batch, const void *Gs, const void *As, const void *x, const void *y,
-                         const void *z, const void *s, const void *exitflag)
+                         const void *z, const void *s, const void *exitflag, const char *fn = "eicos_batch_adjoint")
 {
     if (!bt || batch <= 0)
-        return fail(EICOS_ERR_INVALID, "eicos_batch_adjoint: null handle or batch <= 0");
+        return fail(EICOS_ERR_INVALID, std::string(fn) + ": null handle or batch <= 0");
     if ((Gs || As) && !bt->eng->instance_matrices())
-        return fail(EICOS_ERR_INVALID, "eicos_batch_adjoint: Gs / As need a handle from eicos_batch_setup_ex(..., EICOS_BATCH_INSTANCE_MATRICES)");
+        return fail(EICOS_ERR_INVALID, std::string(fn) + ": Gs / As need a handle from eicos_batch_setup_ex(..., EICOS_BATCH_INSTANCE_MATRICES)");
     const Symbolic &S = bt->S;
     if ((!x && S.n) || (!y && S.p) || (!z && S.m) || (!s && S.m) || !exitflag)
-        return fail(EICOS_ERR_INVALID, "eicos_batch_adjoint: x, y, z, s and exitflag are required");
+        return fail(EICOS_ERR_INVALID, std::string(fn) + ": x, y, z, s and exitflag are required");
     return 0;
 }
 
@@ -492,6 +492,104 @@ int eicos_batch_adjoint(eicos_batch *bt, int batch, const double *Gs, const doub
             be::d2h(db ? db + first * p : nullptr, odb, ob * sizeof(double), st);
             be::d2h(dG ? dG + first * nG : nullptr, odG, oG * sizeof(double), st);
             be::d2h(dA ? dA + first * nA : nullptr, odA, oA * sizeof(double), st);
+            be::d2h(status ? status + first : nullptr, dst, (status ? B : 0) * sizeof(int), st);
+            be::sync(st);
+        }
+        return 0;
+    }
+    catch (const std::invalid_argument &e)
+    {
+        return fail(EICOS_ERR_INVALID, e.what());
+    }
+    catch (const std::exception &e)
+    {
+        return fail(EICOS_ERR_DEVICE, e.what());
+    }
+}
+
+int eicos_batch_tangent_device(eicos_batch *bt, int batch, const double *d_Gs, const double *d_As,
+                               const double *d_x, const double *d_y, const double *d_z, const double *d_s,
+                               const int *d_exitflag, const double *d_dc, const double *d_dh, const double *d_db,
+                               const double *d_dG, const double *d_dA,
+                               double *d_dx, double *d_dy, double *d_dz, double *d_ds, int *d_status)
+{
+    if (const int rc = adjoint_check(bt, batch, d_Gs, d_As, d_x, d_y, d_z, d_s, d_exitflag, "eicos_batch_tangent"))
+        return rc;
+    try
+    {
+        if (bt->eng->instance_matrices())
+            bt->eng->set_matrices(d_Gs, d_As, bt->rawG.data(), bt->rawA.data());
+        bt->eng->tangent(batch, d_x, d_y, d_z, d_s, d_exitflag, d_dc, d_dh, d_db, d_dG, d_dA, d_dx, d_dy, d_dz, d_ds, d_status);
+        return 0;
+    }
+    catch (const std::invalid_argument &e)
+    {
+        return fail(EICOS_ERR_INVALID, e.what());
+    }
+    catch (const std::exception &e)
+    {
+        return fail(EICOS_ERR_DEVICE, e.what());
+    }
+}
+
+int eicos_batch_tangent(eicos_batch *bt, int batch, const double *Gs, const double *As,
+                        const double *x, const double *y, const double *z, const double *s, const int *exitflag,
+                        const double *dc, const double *dh, const double *db, const double *dG, const double *dA,
+                        double *dx, double *dy, double *dz, double *ds, int *status)
+{
+    if (const int rc = adjoint_check(bt, batch, Gs, As, x, y, z, s, exitflag, "eicos_batch_tangent"))
+        return rc;
+    try
+    {
+        const Symbolic &S = bt->S;
+        be::set_device(bt->device);
+        be::stream_t st = (be::stream_t)(intptr_t)bt->eng->stream();
+        // segments of at most `capacity` instances, as in eicos_batch_adjoint: staging bounded by the handle
+        const size_t cap = (size_t)std::max<long long>(1, bt->eng->capacity());
+        const size_t n = S.n, m = S.m, p = S.p, nG = S.G.nnz(), nA = S.A.nnz();
+        for (size_t first = 0; first < (size_t)batch; first += cap)
+        {
+            const size_t B = std::min(cap, (size_t)batch - first);
+            if (bt->eng->instance_matrices())
+            {
+                const size_t ng = Gs ? B * nG : 0, na = As ? B * nA : 0;
+                bt->dmat.ensure((ng + na) * sizeof(double));
+                double *dm = (double *)bt->dmat.p;
+                be::h2d(dm, Gs ? Gs + first * nG : nullptr, ng * sizeof(double), st);
+                be::h2d(dm + ng, As ? As + first * nA : nullptr, na * sizeof(double), st);
+                bt->eng->set_matrices(Gs ? dm : nullptr, As ? dm + ng : nullptr, bt->rawG.data(), bt->rawA.data());
+            }
+            // inputs: x, y, z, s, then the direction components that are given
+            const size_t ix = B * n, iy = B * p, iz = B * m;
+            const size_t jc = dc ? ix : 0, jb = db ? iy : 0, jh = dh ? iz : 0, jG = dG ? B * nG : 0, jA = dA ? B * nA : 0;
+            bt->din.ensure((ix + iy + 2 * iz + jc + jb + jh + jG + jA) * sizeof(double));
+            double *di = (double *)bt->din.p;
+            double *dx_ = di, *dy_ = dx_ + ix, *dz_ = dy_ + iy, *ds_ = dz_ + iz, *ddc = ds_ + iz, *ddb = ddc + jc, *ddh = ddb + jb;
+            double *ddG = ddh + jh, *ddA = ddG + jG;
+            be::h2d(dx_, x ? x + first * n : nullptr, ix * sizeof(double), st);
+            be::h2d(dy_, y ? y + first * p : nullptr, iy * sizeof(double), st);
+            be::h2d(dz_, z ? z + first * m : nullptr, iz * sizeof(double), st);
+            be::h2d(ds_, s ? s + first * m : nullptr, iz * sizeof(double), st);
+            be::h2d(ddc, dc ? dc + first * n : nullptr, jc * sizeof(double), st);
+            be::h2d(ddb, db ? db + first * p : nullptr, jb * sizeof(double), st);
+            be::h2d(ddh, dh ? dh + first * m : nullptr, jh * sizeof(double), st);
+            be::h2d(ddG, dG ? dG + first * nG : nullptr, jG * sizeof(double), st);
+            be::h2d(ddA, dA ? dA + first * nA : nullptr, jA * sizeof(double), st);
+            // outputs that are wanted
+            const size_t ox = dx ? ix : 0, oy = dy ? iy : 0, oz = dz ? iz : 0, os = ds ? iz : 0;
+            bt->dout.ensure((ox + oy + oz + os) * sizeof(double));
+            double *dout = (double *)bt->dout.p;
+            double *odx = dout, *ody = odx + ox, *odz = ody + oy, *ods = odz + oz;
+            bt->dint.ensure(2 * B * sizeof(int));
+            int *dex = (int *)bt->dint.p, *dst = dex + B;
+            be::h2d(dex, exitflag + first, B * sizeof(int), st);
+            bt->eng->tangent((int)B, dx_, dy_, dz_, ds_, dex, dc ? ddc : nullptr, dh ? ddh : nullptr, db ? ddb : nullptr,
+                             dG ? ddG : nullptr, dA ? ddA : nullptr, dx ? odx : nullptr, dy ? ody : nullptr,
+                             dz ? odz : nullptr, ds ? ods : nullptr, dst);
+            be::d2h(dx ? dx + first * n : nullptr, odx, ox * sizeof(double), st);
+            be::d2h(dy ? dy + first * p : nullptr, ody, oy * sizeof(double), st);
+            be::d2h(dz ? dz + first * m : nullptr, odz, oz * sizeof(double), st);
+            be::d2h(ds ? ds + first * m : nullptr, ods, os * sizeof(double), st);
             be::d2h(status ? status + first : nullptr, dst, (status ? B : 0) * sizeof(int), st);
             be::sync(st);
         }

@@ -56,9 +56,10 @@ EI_DEFINE_KERNEL(eicos_debug_line_search, tile_debug_line_search, 2)
 #define EI_LAUNCH_JOBS(name, fn, tiles, njobs, threads, smem, stream, args) \
     name<<<(tiles) * (njobs), (threads), (smem), (stream)>>>(args)
 
-/* adjoint (Engine::adjoint): vector kernels with a second parameter block for the caller's pointers */
-#define EI_DEFINE_ADJ_KERNEL(name, fn)                                                                                   \
-    __global__ void __launch_bounds__(EI_MAX_THREADS, 2) name(const __grid_constant__ KArgs a, const __grid_constant__ AdjArgs g) \
+/* adjoint and tangent (Engine::adjoint, Engine::tangent): vector kernels with a second parameter block for the caller's
+   pointers; the tangent's staging buffers follow the reduction rows (tm.pbuf) */
+#define EI_DEFINE_DIFF_KERNEL(name, fn, Args)                                                                            \
+    __global__ void __launch_bounds__(EI_MAX_THREADS, 2) name(const __grid_constant__ KArgs a, const __grid_constant__ Args g) \
     {                                                                                                                      \
         extern __shared__ double smem[];                                                                                   \
         Team tm;                                                                                                           \
@@ -71,9 +72,11 @@ EI_DEFINE_KERNEL(eicos_debug_line_search, tile_debug_line_search, 2)
         tm.job = 0;                                                                                                        \
         fn(tm, a, g, (int)blockIdx.x);                                                                                     \
     }
-EI_DEFINE_ADJ_KERNEL(eicos_adjoint_load, tile_adjoint_load)
-EI_DEFINE_ADJ_KERNEL(eicos_adjoint_store, tile_adjoint_store)
-#define EI_LAUNCH_ADJ(name, fn, tiles, threads, smem, stream, args, adj) name<<<(tiles), (threads), (smem), (stream)>>>(args, adj)
+EI_DEFINE_DIFF_KERNEL(eicos_adjoint_load, tile_adjoint_load, AdjArgs)
+EI_DEFINE_DIFF_KERNEL(eicos_adjoint_store, tile_adjoint_store, AdjArgs)
+EI_DEFINE_DIFF_KERNEL(eicos_tangent_load, tile_tangent_load, TanArgs)
+EI_DEFINE_DIFF_KERNEL(eicos_tangent_store, tile_tangent_store, TanArgs)
+#define EI_LAUNCH_DIFF(name, fn, tiles, threads, smem, stream, args, extra) name<<<(tiles), (threads), (smem), (stream)>>>(args, extra)
 
 __global__ void eicos_compact(const __grid_constant__ KArgs a, const __grid_constant__ MoveRanges mr, const int *moves)
 {
@@ -120,11 +123,17 @@ __global__ void eicos_compact(const __grid_constant__ KArgs a, const __grid_cons
 #endif
 
 #ifdef EICOS_EMU
-#define EI_LAUNCH_ADJ(name, fn, tiles, threads, smem, stream, args, adj)                                    \
-    do                                                                                                      \
-    {                                                                                                       \
-        const auto fn_ = [&](const Team &tm_, const KArgs &a_, int tile_) { fn(tm_, a_, (adj), tile_); }; \
-        EI_LAUNCH(name, fn_, tiles, threads, smem, stream, args);                                           \
+// (every CTA gets staging buffers for its workers in pbuf, as the device kernels do after the reduction rows)
+#define EI_LAUNCH_DIFF(name, fn, tiles, threads, smem, stream, args, extra)                      \
+    do                                                                                           \
+    {                                                                                            \
+        std::vector<double> stage_((size_t)(threads) * TAN_STAGE_DOUBLES);                       \
+        const auto fn_ = [&](const Team &tm_, const KArgs &a_, int tile_) {                      \
+            Team t2_ = tm_;                                                                      \
+            t2_.pbuf = stage_.data();                                                            \
+            fn(t2_, a_, (extra), tile_);                                                         \
+        };                                                                                       \
+        EI_LAUNCH(name, fn_, tiles, threads, smem, stream, args);                                \
     } while (0)
 #endif
 
@@ -287,19 +296,21 @@ void Engine::upload_pattern(const Symbolic &S)
     P.pim = pim_ ? 1 : 0;
     P.nnzG = S.G.nnz();
     P.nnzA = S.A.nnz();
-    // CSC index arrays of G and A: the on-device equilibration and the adjoint's per-entry gradients walk them
+    // CSC index arrays of G and A: the on-device equilibration, the adjoint's per-entry gradients and the tangent's
+    // column products walk them
     P.Gp = upload(S.G.p, owned_, st);
     P.Gi = upload(S.G.i, owned_, st);
     P.Ap = upload(S.A.p, owned_, st);
     P.Ai = upload(S.A.i, owned_, st);
+    // their CSR views (row pointers, value slots, columns): the on-device equilibration and the tangent's row products
+    P.Grp = upload(S.Gr.p, owned_, st);
+    P.Grv = upload(S.Gr.v, owned_, st);
+    P.Arp = upload(S.Ar.p, owned_, st);
+    P.Arv = upload(S.Ar.v, owned_, st);
+    dGrj_ = upload(S.Gr.j, owned_, st);
+    dArj_ = upload(S.Ar.j, owned_, st);
     if (pim_)
-    {
-        P.Grp = upload(S.Gr.p, owned_, st);
-        P.Grv = upload(S.Gr.v, owned_, st);
-        P.Arp = upload(S.Ar.p, owned_, st);
-        P.Arv = upload(S.Ar.v, owned_, st);
         P.cone_z = upload(S.cone_z, owned_, st);
-    }
     P.cone_dim = upload(S.q, owned_, st);
     P.cone_k = upload(S.cone_k, owned_, st);
     P.cone_q = upload(S.cone_q, owned_, st);
@@ -467,6 +478,7 @@ Engine::Engine(const Symbolic &S, int device, long long capacity_instances, int 
                   std::max((size_t)M_MV_PARTS * part_doubles_, std::max(smem_prog_[0], smem_prog_[M_VARIANTS - 1]) / sizeof(double))) *
                  sizeof(double);
     smem_common_ = workers_ > 1 ? (size_t)workers_ * KRED * TILE * sizeof(double) : 0;
+    smem_tangent_ = (size_t)workers_ * (KRED * TILE + TAN_STAGE_DOUBLES) * sizeof(double);
 #ifndef EICOS_EMU
     {
         if (smem_pair_ > 48 * 1024)
@@ -495,10 +507,13 @@ Engine::Engine(const Symbolic &S, int device, long long capacity_instances, int 
         const void *ks[] = {(const void *)eicos_load_inputs, (const void *)eicos_equilibrate, (const void *)eicos_init,
                             (const void *)eicos_init_point,
                             (const void *)eicos_iter_head, (const void *)eicos_iter_mid, (const void *)eicos_iter_tail,
-                            (const void *)eicos_store_outputs, (const void *)eicos_adjoint_load, (const void *)eicos_adjoint_store};
+                            (const void *)eicos_store_outputs, (const void *)eicos_adjoint_load, (const void *)eicos_adjoint_store,
+                            (const void *)eicos_tangent_store};
         for (const void *k : ks)
             EI_CUDA(cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_common_));
     }
+    if (smem_tangent_ > 48 * 1024)
+        EI_CUDA(cudaFuncSetAttribute(eicos_tangent_load, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_tangent_));
 #endif
     be::sync(S_(stream_));
 }
@@ -882,16 +897,8 @@ void Engine::solve(int batch, const double *d_c, const double *d_h, const double
 #undef EI_TIMED
 }
 
-void Engine::adjoint(int batch, const double *d_x, const double *d_y, const double *d_z, const double *d_s, const int *d_exit,
-                     const double *d_gx, const double *d_gy, const double *d_gz,
-                     double *d_dc, double *d_dh, double *d_db, double *d_dG, double *d_dA, int *d_status)
+KArgs Engine::diff_args()
 {
-    be::set_device(device_);
-    be::stream_t st = S_(stream_);
-    if (batch <= 0)
-        return;
-    if ((!d_x && P_.n) || (!d_y && P_.p) || (!d_z && P_.m) || (!d_s && P_.m) || !d_exit)
-        throw std::invalid_argument("adjoint: x, y, z, s and the exit flags are required");
     KArgs a;
     std::memset(&a, 0, sizeof(a));
     a.P = P_;
@@ -903,7 +910,7 @@ void Engine::adjoint(int batch, const double *d_x, const double *d_y, const doub
     a.part_doubles = (int)part_doubles_;
     if (pim_)
     { // eicos_load_inputs brings this chunk's matrices (and vectors nobody reads here: zeros)
-        be::zero(base_vec_, (size_t)(P_.n + P_.m + P_.p) * sizeof(double), st);
+        be::zero(base_vec_, (size_t)(P_.n + P_.m + P_.p) * sizeof(double), S_(stream_));
         a.base_c = base_vec_;
         a.base_h = base_vec_ + P_.n;
         a.base_b = base_vec_ + P_.n + P_.m;
@@ -912,15 +919,49 @@ void Engine::adjoint(int batch, const double *d_x, const double *d_y, const doub
         a.base_G = base_mat_;
         a.base_A = base_mat_ + nnzG_;
     }
+    return a;
+}
+
+// the factorisation at the scalings the load step wrote, and one solveKKT (rhs1 -> sol1) in the form and ring depth a
+// one-job solve of the iteration takes
+void Engine::factor_solve(KArgs &a, int tiles)
+{
+    be::stream_t st = S_(stream_);
+    const int threads1 = LANES == 1 ? 1 : 32, threads_wide = M_MV_PARTS * (LANES == 1 ? 1 : 32);
+    (void)threads1;
+    (void)threads_wide;
+    (void)st;
+    a.variant = deep_ring(tiles) ? M_VARIANTS - 1 : 0;
+    EI_LAUNCH(eicos_ldl_factor, tile_factor, tiles, threads1, smem_factor_[a.variant], st, a);
+    a.job[0] = {L_.rhs1, L_.sol1, J_NIT1, 0};
+    a.initialize = 0;
+    a.variant = deep_ring(tiles) ? M_VARIANTS - 1 : 0;
+    if (wide_launch(tiles))
+    {
+        a.variant = force_variant_ == 0 ? 0 : M_VARIANTS - 1;
+        EI_LAUNCH_JOBS(eicos_solve_kkt_wide, tile_solve_kkt<1>, tiles, 1, threads_wide, smem_wide_, st, a);
+    }
+    else
+        EI_LAUNCH_JOBS(eicos_solve_kkt, tile_solve_kkt<1>, tiles, 1, threads1, smem_prog_[a.variant], st, a);
+}
+
+void Engine::adjoint(int batch, const double *d_x, const double *d_y, const double *d_z, const double *d_s, const int *d_exit,
+                     const double *d_gx, const double *d_gy, const double *d_gz,
+                     double *d_dc, double *d_dh, double *d_db, double *d_dG, double *d_dA, int *d_status)
+{
+    be::set_device(device_);
+    be::stream_t st = S_(stream_);
+    if (batch <= 0)
+        return;
+    if ((!d_x && P_.n) || (!d_y && P_.p) || (!d_z && P_.m) || (!d_s && P_.m) || !d_exit)
+        throw std::invalid_argument("adjoint: x, y, z, s and the exit flags are required");
+    KArgs a = diff_args();
     AdjArgs g;
     g.x = d_x, g.y = d_y, g.z = d_z, g.s = d_s, g.exit = d_exit;
     g.gx = d_gx, g.gy = d_gy, g.gz = d_gz;
     g.dc = d_dc, g.dh = d_dh, g.db = d_db, g.dG = d_dG, g.dA = d_dA, g.status = d_status;
-    const int threads = workers_ * (LANES == 1 ? 1 : 32), threads1 = LANES == 1 ? 1 : 32;
-    const int threads_wide = M_MV_PARTS * (LANES == 1 ? 1 : 32);
+    const int threads = workers_ * (LANES == 1 ? 1 : 32);
     (void)threads;
-    (void)threads1;
-    (void)threads_wide;
     for (long long first = 0; first < batch; first += cap_tiles_ * TILE)
     {
         const int nb = (int)std::min<long long>(batch - first, cap_tiles_ * TILE);
@@ -932,21 +973,51 @@ void Engine::adjoint(int batch, const double *d_x, const double *d_y, const doub
             EI_LAUNCH(eicos_load_inputs, tile_load, tiles, threads, smem_common_, st, a);
             EI_LAUNCH(eicos_equilibrate, tile_equil, tiles, threads, smem_common_, st, a);
         }
-        EI_LAUNCH_ADJ(eicos_adjoint_load, tile_adjoint_load, tiles, threads, smem_common_, st, a, g);
-        a.variant = deep_ring(tiles) ? M_VARIANTS - 1 : 0;
-        EI_LAUNCH(eicos_ldl_factor, tile_factor, tiles, threads1, smem_factor_[a.variant], st, a);
-        // one solveKKT (rhs1 -> sol1) in the form and ring depth a one-job solve of the iteration takes
-        a.job[0] = {L_.rhs1, L_.sol1, J_NIT1, 0};
-        a.initialize = 0;
-        a.variant = deep_ring(tiles) ? M_VARIANTS - 1 : 0;
-        if (wide_launch(tiles))
+        EI_LAUNCH_DIFF(eicos_adjoint_load, tile_adjoint_load, tiles, threads, smem_common_, st, a, g);
+        factor_solve(a, tiles);
+        EI_LAUNCH_DIFF(eicos_adjoint_store, tile_adjoint_store, tiles, threads, smem_common_, st, a, g);
+    }
+#ifndef EICOS_EMU
+    EI_CUDA(cudaGetLastError());
+#endif
+    be::sync(st);
+}
+
+void Engine::tangent(int batch, const double *d_x, const double *d_y, const double *d_z, const double *d_s, const int *d_exit,
+                     const double *d_dc, const double *d_dh, const double *d_db, const double *d_dG, const double *d_dA,
+                     double *d_ox, double *d_oy, double *d_oz, double *d_os, int *d_status)
+{
+    be::set_device(device_);
+    be::stream_t st = S_(stream_);
+    if (batch <= 0)
+        return;
+    if ((!d_x && P_.n) || (!d_y && P_.p) || (!d_z && P_.m) || (!d_s && P_.m) || !d_exit)
+        throw std::invalid_argument("tangent: x, y, z, s and the exit flags are required");
+    // the load step stages dG / dA in the rows of L (every entry of G and A is an entry of L's pattern)
+    if ((d_dG || d_dA) && P_.nnzL < P_.nnzG + P_.nnzA)
+        throw std::runtime_error("tangent: the factor has fewer entries than G and A together");
+    KArgs a = diff_args();
+    TanArgs g;
+    g.x = d_x, g.y = d_y, g.z = d_z, g.s = d_s, g.exit = d_exit;
+    g.dc = d_dc, g.dh = d_dh, g.db = d_db, g.dG = d_dG, g.dA = d_dA;
+    g.dx = d_ox, g.dy = d_oy, g.dz = d_oz, g.ds = d_os, g.status = d_status;
+    g.Grj = dGrj_, g.Arj = dArj_;
+    const int threads = workers_ * (LANES == 1 ? 1 : 32);
+    (void)threads;
+    for (long long first = 0; first < batch; first += cap_tiles_ * TILE)
+    {
+        const int nb = (int)std::min<long long>(batch - first, cap_tiles_ * TILE);
+        const int tiles = (nb + TILE - 1) / TILE;
+        a.batch = nb;
+        a.first = (int)first;
+        if (pim_)
         {
-            a.variant = force_variant_ == 0 ? 0 : M_VARIANTS - 1;
-            EI_LAUNCH_JOBS(eicos_solve_kkt_wide, tile_solve_kkt<1>, tiles, 1, threads_wide, smem_wide_, st, a);
+            EI_LAUNCH(eicos_load_inputs, tile_load, tiles, threads, smem_common_, st, a);
+            EI_LAUNCH(eicos_equilibrate, tile_equil, tiles, threads, smem_common_, st, a);
         }
-        else
-            EI_LAUNCH_JOBS(eicos_solve_kkt, tile_solve_kkt<1>, tiles, 1, threads1, smem_prog_[a.variant], st, a);
-        EI_LAUNCH_ADJ(eicos_adjoint_store, tile_adjoint_store, tiles, threads, smem_common_, st, a, g);
+        EI_LAUNCH_DIFF(eicos_tangent_load, tile_tangent_load, tiles, threads, smem_tangent_, st, a, g);
+        factor_solve(a, tiles);
+        EI_LAUNCH_DIFF(eicos_tangent_store, tile_tangent_store, tiles, threads, smem_common_, st, a, g);
     }
 #ifndef EICOS_EMU
     EI_CUDA(cudaGetLastError());

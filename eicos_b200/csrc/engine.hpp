@@ -13,6 +13,8 @@
 namespace eicos
 {
 
+struct KArgs; // tile_program.hpp
+
 struct SolveStats
 {
     int chunks = 0, compactions = 0;
@@ -92,6 +94,15 @@ class Engine
                  const double *d_gx, const double *d_gy, const double *d_gz,
                  double *d_dc, double *d_dh, double *d_db, double *d_dG, double *d_dA, int *d_status);
 
+    // Derivatives of the solution map along a direction v = (dc, dh, db, dG, dA) for `batch` instances: the same
+    // factorisation and solveKKT as adjoint(), with K0 [dx; dy; dz] = [-dc - dA'y - dG'z; db - dA x; dh - dG x] and
+    // ds = -W^2 dz.  d_x .. d_exit: the forward's results; d_dc .. d_dA: the direction (null = zero; dG / dA
+    // [batch x nnzG / nnzA] in CSC order, on either kind of handle); outputs dx [batch x n], dy [batch x p],
+    // dz, ds [batch x m], status [batch] (any may be null).  Layouts as in adjoint().  Blocks until done.
+    void tangent(int batch, const double *d_x, const double *d_y, const double *d_z, const double *d_s, const int *d_exit,
+                 const double *d_dc, const double *d_dh, const double *d_db, const double *d_dG, const double *d_dA,
+                 double *d_dx, double *d_dy, double *d_dz, double *d_ds, int *d_status);
+
     // debug entry points (GPU unit tests): run the initial factorisation / one KKT solve for
     // instance-major data and copy raw factor values back (host pointers, may be null)
     void debug_factor_init(int batch, const double *d_c, const double *d_h, const double *d_b,
@@ -120,6 +131,8 @@ class Engine
   private:
     void build_layout(const Symbolic &S, bool acc_rows);
     void upload_pattern(const Symbolic &S);
+    KArgs diff_args();                      // adjoint / tangent: the kernel arguments of every chunk
+    void factor_solve(KArgs &a, int tiles); // adjoint / tangent: factorisation + one solveKKT (rhs1 -> sol1)
 
     int device_ = 0, workers_ = 4;
     bool pim_ = false;
@@ -141,6 +154,8 @@ class Engine
     bool compaction_ = true;
     size_t smem_factor_[M_VARIANTS] = {0, 0}, smem_common_ = 0, smem_prog_[M_VARIANTS] = {0, 0}; // factor kernel / vector kernels / solveKKT + residual kernels (per ring variant)
     size_t smem_pair_ = 0; // two-job solveKKT kernel
+    size_t smem_tangent_ = 0; // eicos_tangent_load: reduction rows + one staging buffer per worker
+    const int *dGrj_ = nullptr, *dArj_ = nullptr; // columns of the CSR views of G and A (the tangent's row products)
     size_t smem_resid_ = 0, smem_wide_ = 0, part_doubles_ = 0; // one-warp residual kernel; wide kernels; one part machine (doubles)
     int force_wide_ = -1;
     KSettings settings_ = default_settings();

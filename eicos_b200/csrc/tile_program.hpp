@@ -2762,6 +2762,136 @@ EI_DEV vd adj_eq(const KArgs &a, const double *T, int q)
     return vset(q < n ? EI_LDG(a.P.xeq + q) : (q < zb ? EI_LDG(a.P.Aeq + q - n) : EI_LDG(a.P.GeqE + q - zb)));
 }
 
+// ---- shared by the adjoint and the tangent: both differentiate through the same K0 at the forward's (s, z)
+// the chunk's instances of this lane: valid (not padding) and global index within the device batch
+EI_DEV void diff_lanes(const Team &tm, const KArgs &a, int tile, bool (&valid)[VEC], size_t (&gi)[VEC])
+{
+    VFOR
+    {
+        int inst = tile * TILE + tm.lane + c_;
+        valid[c_] = inst < a.batch;
+        if (!valid[c_])
+            inst = a.batch - 1; // padding lanes replay the last instance; nothing of theirs is stored
+        gi[c_] = (size_t)a.first + inst;
+    }
+}
+
+// the two expansion slots of every cone: zero in every z-shaped row the solve reads
+EI_DEV void diff_zero_slots(const Team &tm, const KArgs &a, double *T)
+{
+    const DevPattern &P = a.P;
+    const Layout &L = a.L;
+    const int zb = P.n + P.p;
+    for (int c = tm.wk; c < P.nc; c += tm.nwk)
+    {
+        const int e = EI_LDG(P.cone_k + c) + EI_LDG(P.cone_dim + c);
+        for (int k = e; k < e + 2; k++)
+        {
+            ROWD(T, L.w + zb + k) = 0.0;
+            ROWD(T, L.s + k) = 0.0;
+            ROWD(T, L.lam + k) = 0.0;
+            ROWD(T, L.rhs1 + zb + k) = 0.0;
+        }
+    }
+}
+
+// After the rows s = s_e and lam = z_e are written (this begins with a barrier): updateScalings (src/eicos.cpp:411-479)
+// of (s_e, z_e) into the scaling rows, updateKKTScalings (:1691-1732) into the V block, and red[1] = 1 for an
+// instance not strictly interior.  red[0] (max |rhs1|) and red[1] are combined over the workers.
+EI_DEV void diff_scalings(const Team &tm, const KArgs &a, double *T, vd (&red)[2])
+{
+    const DevPattern &P = a.P;
+    const Layout &L = a.L;
+    tm.sync(); // the rows above are complete before the passes below, which split them differently
+    for (int k = tm.wk; k < P.l; k += tm.nwk)
+    {
+        const vd sv = ROWD(T, L.s + k), zv = ROWD(T, L.lam + k);
+        const vd v = sv / zv;
+        ROWD(T, L.lpv + k) = -v;
+        ROWD(T, L.lpw + k) = vsqrt(v);
+        ROWD(T, L.V + k) = -v - Settings::deltastat;
+        VFOR if (!(sv.v[c_] > 0 && zv.v[c_] > 0)) red[1].v[c_] = 1.0;
+    }
+    for (int c = tm.wk; c < P.nc; c += tm.nwk)
+    {
+        const int d = EI_LDG(P.cone_dim + c), ks = EI_LDG(P.cone_k + c), qo = EI_LDG(P.cone_q + c);
+        VFOR
+        {
+            const ConeScaling cs = cone_scaling(tm, T, L.s + ks, L.lam + ks, d, c_);
+            if (cs.stage != 0)
+                red[1].v[c_] = 1.0;
+            else
+                cone_scaling_rows(T, L, L.cpar + c * CP_COUNT, qo, L.s + ks, L.lam + ks, d, cs, c_);
+        }
+    }
+    team_max<2>(tm, red);
+    cone_kkt_scalings(tm, a, T); // (cone c's scaling rows were written by this worker)
+}
+
+// The lanes to differentiate stay ST_ACTIVE, so that the factorisation and solveKKT run on them only; every other
+// lane is frozen with its ADJ_* status (exit flag first, then interiority).  red: max |rhs1|, "not interior".
+EI_DEV void diff_status(const Team &tm, const KArgs &a, const TileMem &t, const int *exit, const bool (&valid)[VEC],
+                        const size_t (&gi)[VEC], const vd (&red)[2])
+{
+    if (tm.wk == 0)
+        VFOR
+        {
+            const int ex = exit[gi[c_]];
+            const int st = ex != EXIT_OPTIMAL && ex != EXIT_OPTIMAL + EXIT_INACC ? ADJ_NOT_OPTIMAL
+                           : red[1].v[c_] != 0.0                               ? ADJ_NOT_INTERIOR
+                                                                               : (int)ST_ACTIVE;
+            ROWC(t.I, J_STATUS, c_) = valid[c_] ? st : (int)EXIT_FATAL;
+            ROWC(t.I, J_INST, c_) = valid[c_] ? (int)gi[c_] : -1;
+            ROWC(t.T, a.L.sc + S_RHSMAX1, c_) = red[0].v[c_];
+        }
+}
+
+// After solveKKT (rhs1 -> sol1): rows dst = D^-1 sol1 (the solution in the original scaling), the final status of
+// every lane (ADJ_NOT_FINITE when a value is not finite) and the mask of the lanes that were differentiated.
+EI_DEV void diff_unscale(const Team &tm, const KArgs &a, const TileMem &t, int dst, int (&code)[VEC], vb &diff)
+{
+    const Layout &L = a.L;
+    double *T = t.T;
+    VFOR diff.v[c_] = ROWC(t.I, J_STATUS, c_) == ST_ACTIVE;
+    vd bad[1] = {vset(0.0)};
+    for (int q = tm.wk; q < a.P.N; q += tm.nwk)
+    {
+        const vd u = vd(ROWD(T, L.sol1 + q)) / adj_eq(a, T, q);
+        ROWD(T, dst + q) = u;
+        VFOR if (!(fabs(u.v[c_]) <= DBL_MAX)) bad[0].v[c_] = 1.0;
+    }
+    team_max<1>(tm, bad); // (its barriers also complete the rows before the passes below)
+    VFOR
+    {
+        const int st = ROWC(t.I, J_STATUS, c_);
+        code[c_] = st == ST_ACTIVE ? (bad[0].v[c_] != 0.0 ? ADJ_NOT_FINITE : ADJ_OK) : (st == EXIT_FATAL ? ADJ_NOT_FINITE : st);
+        diff.v[c_] = diff.v[c_] && code[c_] == ADJ_OK;
+    }
+}
+
+// out[inst * stride + k] = v for this lane's instances; exact zeros for a lane not differentiated
+EI_DEV void diff_put(const TileMem &t, vb diff, double *out, int stride, int k, vd v)
+{
+    v = vsel(diff, v, vset(0.0));
+    VFOR
+    {
+        const int inst = ROWC(t.I, J_INST, c_);
+        if (inst >= 0)
+            out[(size_t)inst * stride + k] = v.v[c_];
+    }
+}
+
+EI_DEV void diff_write_status(const Team &tm, const TileMem &t, int *status, const int (&code)[VEC])
+{
+    if (tm.wk == 0 && status)
+        VFOR
+        {
+            const int inst = ROWC(t.I, J_INST, c_);
+            if (inst >= 0)
+                status[inst] = code[c_];
+        }
+}
+
 // Loads the iterate and the incoming gradients of the chunk's instances, builds the Nesterov-Todd scalings of the
 // equilibrated (s, z) into the scaling rows and the V block (what the head step's updateScalings / updateKKTScalings
 // write), and rhs1 = D^-1 [gx; gy; gz] with D = diag(x_equil, A_equil, G_equil).  The lanes to differentiate are
@@ -2776,14 +2906,7 @@ EI_DEV void tile_adjoint_load(const Team &tm, const KArgs &a, const AdjArgs &g, 
     const int n = P.n, zb = P.n + P.p;
     bool valid[VEC];
     size_t gi[VEC];
-    VFOR
-    {
-        int inst = tile * TILE + tm.lane + c_;
-        valid[c_] = inst < a.batch;
-        if (!valid[c_])
-            inst = a.batch - 1; // padding lanes replay the last instance; nothing of theirs is stored
-        gi[c_] = (size_t)a.first + inst;
-    }
+    diff_lanes(tm, a, tile, valid, gi);
     vd red[2] = {vset(0.0), vset(0.0)}; // max |rhs1|, "not interior"
     for (int j = tm.wk; j < n; j += tm.nwk)
     {
@@ -2828,53 +2951,9 @@ EI_DEV void tile_adjoint_load(const Team &tm, const KArgs &a, const AdjArgs &g, 
         ROWD(T, L.rhs1 + zb + e) = r;
         red[0] = vmax(red[0], vabs(r));
     }
-    for (int c = tm.wk; c < P.nc; c += tm.nwk)
-    { // the two expansion slots of every cone: zero in every z-shaped row
-        const int e = EI_LDG(P.cone_k + c) + EI_LDG(P.cone_dim + c);
-        for (int k = e; k < e + 2; k++)
-        {
-            ROWD(T, L.w + zb + k) = 0.0;
-            ROWD(T, L.s + k) = 0.0;
-            ROWD(T, L.lam + k) = 0.0;
-            ROWD(T, L.rhs1 + zb + k) = 0.0;
-        }
-    }
-    tm.sync(); // the rows above are complete before the passes below, which split them differently
-    // updateScalings (src/eicos.cpp:411-479) of (s_e, z_e) and updateKKTScalings (:1691-1732)
-    for (int k = tm.wk; k < P.l; k += tm.nwk)
-    {
-        const vd sv = ROWD(T, L.s + k), zv = ROWD(T, L.lam + k);
-        const vd v = sv / zv;
-        ROWD(T, L.lpv + k) = -v;
-        ROWD(T, L.lpw + k) = vsqrt(v);
-        ROWD(T, L.V + k) = -v - Settings::deltastat;
-        VFOR if (!(sv.v[c_] > 0 && zv.v[c_] > 0)) red[1].v[c_] = 1.0;
-    }
-    for (int c = tm.wk; c < P.nc; c += tm.nwk)
-    {
-        const int d = EI_LDG(P.cone_dim + c), ks = EI_LDG(P.cone_k + c), qo = EI_LDG(P.cone_q + c);
-        VFOR
-        {
-            const ConeScaling cs = cone_scaling(tm, T, L.s + ks, L.lam + ks, d, c_);
-            if (cs.stage != 0)
-                red[1].v[c_] = 1.0;
-            else
-                cone_scaling_rows(T, L, L.cpar + c * CP_COUNT, qo, L.s + ks, L.lam + ks, d, cs, c_);
-        }
-    }
-    team_max<2>(tm, red);
-    cone_kkt_scalings(tm, a, T); // (cone c's scaling rows were written by this worker)
-    if (tm.wk == 0)
-        VFOR
-        {
-            const int ex = g.exit[gi[c_]];
-            const int st = ex != EXIT_OPTIMAL && ex != EXIT_OPTIMAL + EXIT_INACC ? ADJ_NOT_OPTIMAL
-                           : red[1].v[c_] != 0.0                               ? ADJ_NOT_INTERIOR
-                                                                               : (int)ST_ACTIVE;
-            ROWC(t.I, J_STATUS, c_) = valid[c_] ? st : (int)EXIT_FATAL;
-            ROWC(t.I, J_INST, c_) = valid[c_] ? (int)gi[c_] : -1;
-            ROWC(T, L.sc + S_RHSMAX1, c_) = red[0].v[c_];
-        }
+    diff_zero_slots(tm, a, T);
+    diff_scalings(tm, a, T, red);
+    diff_status(tm, a, t, g.exit, valid, gi, red);
 }
 
 // After the factorisation and solveKKT (rhs1 -> sol1): u = D^-1 sol1 solves K0 u = g in the original scaling.
@@ -2889,32 +2968,9 @@ EI_DEV void tile_adjoint_store(const Team &tm, const KArgs &a, const AdjArgs &g,
     double *T = t.T;
     const int n = P.n, zb = P.n + P.p;
     vb diff;
-    VFOR diff.v[c_] = ROWC(t.I, J_STATUS, c_) == ST_ACTIVE;
-    vd bad[1] = {vset(0.0)};
-    for (int q = tm.wk; q < P.N; q += tm.nwk)
-    {
-        const vd u = vd(ROWD(T, L.sol1 + q)) / adj_eq(a, T, q);
-        ROWD(T, L.sol1 + q) = u;
-        VFOR if (!(fabs(u.v[c_]) <= DBL_MAX)) bad[0].v[c_] = 1.0;
-    }
-    team_max<1>(tm, bad); // (its barriers also complete u before the passes below)
     int code[VEC];
-    VFOR
-    {
-        const int st = ROWC(t.I, J_STATUS, c_);
-        code[c_] = st == ST_ACTIVE ? (bad[0].v[c_] != 0.0 ? ADJ_NOT_FINITE : ADJ_OK) : (st == EXIT_FATAL ? ADJ_NOT_FINITE : st);
-        diff.v[c_] = diff.v[c_] && code[c_] == ADJ_OK;
-    }
-    const vd zero = vset(0.0);
-    const auto put = [&](double *out, int stride, int k, vd v) {
-        v = vsel(diff, v, zero);
-        VFOR
-        {
-            const int inst = ROWC(t.I, J_INST, c_);
-            if (inst >= 0)
-                out[(size_t)inst * stride + k] = v.v[c_];
-        }
-    };
+    diff_unscale(tm, a, t, L.sol1, code, diff);
+    const auto put = [&](double *out, int stride, int k, vd v) { diff_put(t, diff, out, stride, k, v); };
     if (g.dc)
         for (int j = tm.wk; j < n; j += tm.nwk)
             put(g.dc, n, j, -vd(ROWD(T, L.sol1 + j)));
@@ -2943,13 +2999,217 @@ EI_DEV void tile_adjoint_store(const Team &tm, const KArgs &a, const AdjArgs &g,
                     put(g.dA, P.nnzA, k, -(vd(ROWD(T, L.w + r)) * uxj + vd(ROWD(T, L.sol1 + r)) * xj));
                 }
         }
-    if (tm.wk == 0 && g.status)
+    diff_write_status(tm, t, g.status, code);
+}
+
+// ------------------------------------------------------------------ tangent of the solution map (Engine::tangent)
+// Pointers of one tangent call: the forward's results and the direction v = (dc, dh, db, dG, dA) in, the derivatives
+// of (x, y, z, s) along v out; instance-major, original scaling, z-shaped arrays in compact z order, dG / dA in CSC
+// order.  A null direction component is zero; any output may be null.  Grj / Arj: column of every entry of the CSR
+// views of G and A (the row pointers and value slots are DevPattern's Grp / Grv / Arp / Arv).
+struct TanArgs
+{
+    const double *x, *y, *z, *s;
+    const int *exit;
+    const double *dc, *dh, *db, *dG, *dA;
+    double *dx, *dy, *dz, *ds;
+    int *status;
+    const int *Grj, *Arj;
+};
+
+constexpr int TAN_RUN = 16;          // consecutive stack entries a warp stages per instance
+constexpr int TAN_LD = TILE + 2;     // row stride (doubles) of a staging buffer: 16-byte rows, two-way bank conflicts
+constexpr int TAN_BATCH = 16;        // loads in flight per lane while staging
+static_assert(TILE * TAN_RUN % (LANES * TAN_BATCH) == 0, "staging batches");
+
+constexpr int TAN_STAGE_DOUBLES = TAN_RUN * TAN_LD; // one worker's staging buffer (tm.pbuf + wk * TAN_STAGE_DOUBLES)
+
+EI_DEV void warp_sync()
+{
+#ifndef EICOS_EMU
+    __syncwarp();
+#endif
+}
+
+// Copies the tile's part of an instance-major stack src [batch x cnt] into the rows row0 .. row0 + cnt - 1.  A worker
+// takes runs of TAN_RUN consecutive entries: its lanes read the run of every instance of the tile with consecutive
+// addresses (TAN_RUN doubles per instance), the warp's shared-memory buffer transposes them, and each lane stores its
+// instances' part of whole rows.  Padding lanes read the last instance, as they do everywhere else.
+EI_DEV void tan_stage(const Team &tm, const KArgs &a, const TileMem &t, int tile, const double *src, int cnt, int row0)
+{
+    double *buf = tm.pbuf + (size_t)tm.wk * TAN_STAGE_DOUBLES;
+    const int last = a.batch - 1;
+    for (int k0 = tm.wk * TAN_RUN; k0 < cnt; k0 += tm.nwk * TAN_RUN)
+    {
+        const int len = cnt - k0 < TAN_RUN ? cnt - k0 : TAN_RUN;
+        for (int f0 = 0; f0 < TILE * TAN_RUN; f0 += LANES * TAN_BATCH)
+        {
+            double v[TAN_BATCH];
+#pragma unroll
+            for (int u = 0; u < TAN_BATCH; u++)
+            {
+                const int f = f0 + u * LANES + tm.pl, i = f / TAN_RUN, o = f % TAN_RUN;
+                const int inst = tile * TILE + i < last ? tile * TILE + i : last;
+                v[u] = o < len ? src[((size_t)a.first + inst) * cnt + k0 + o] : 0.0;
+            }
+#pragma unroll
+            for (int u = 0; u < TAN_BATCH; u++)
+            {
+                const int f = f0 + u * LANES + tm.pl;
+                buf[(f % TAN_RUN) * TAN_LD + f / TAN_RUN] = v[u];
+            }
+        }
+        warp_sync();
+        for (int o = 0; o < len; o++)
+            ROWD(t.T, row0 + k0 + o) = vload(buf + o * TAN_LD + tm.lane);
+        warp_sync(); // the buffer is read before the next run overwrites it
+    }
+}
+
+// Loads the iterate, builds the scalings and the V block as the adjoint does (diff_scalings), and the right-hand side
+//     r = [-dc - dA'y - dG'z;  db - dA x;  dh - dG x],   rhs1 = D^-1 r,   D = diag(x_equil, A_equil, G_equil),
+// from the original x, y, z.  The direction stacks dG / dA are staged into the rows of L (free until the factorisation
+// that follows writes them: Engine::tangent checks nnzL >= nnzG + nnzA).  Summation order, fixed whatever the batch,
+// the chunking or the number of workers: one worker owns a row of r; it starts from the direction term and subtracts
+// the products in ascending CSC position (x rows: the entries of column j of A, then of G) or ascending CSR position
+// (y and z rows), each with one rounding (fma).  A null stack contributes exact zeros through the same operations, so
+// that a null direction gives the bits of a zero one.
+EI_DEV void tile_tangent_load(const Team &tm, const KArgs &a, const TanArgs &g, int tile)
+{
+    const TileMem t = tile_mem(tm, a, tile);
+    const DevPattern &P = a.P;
+    const Layout &L = a.L;
+    double *T = t.T;
+    const int n = P.n, zb = P.n + P.p;
+    bool valid[VEC];
+    size_t gi[VEC];
+    diff_lanes(tm, a, tile, valid, gi);
+    for (int j = tm.wk; j < n; j += tm.nwk)
+    {
+        vd xv;
+        VFOR xv.v[c_] = g.x[gi[c_] * n + j];
+        ROWD(T, L.w + j) = xv;
+    }
+    for (int i = tm.wk; i < P.p; i += tm.nwk)
+    {
+        vd yv;
+        VFOR yv.v[c_] = g.y[gi[c_] * P.p + i];
+        ROWD(T, L.w + n + i) = yv;
+    }
+    for (int i = tm.wk; i < P.m; i += tm.nwk)
+    {
+        const int e = EI_LDG(P.zk + i);
+        vd zv, sv;
         VFOR
         {
-            const int inst = ROWC(t.I, J_INST, c_);
-            if (inst >= 0)
-                g.status[inst] = code[c_];
+            zv.v[c_] = g.z[gi[c_] * P.m + i];
+            sv.v[c_] = g.s[gi[c_] * P.m + i];
         }
+        const vd eq = adj_eq(a, T, zb + e);
+        ROWD(T, L.w + zb + e) = zv;
+        ROWD(T, L.s + e) = sv / eq;
+        ROWD(T, L.lam + e) = zv * eq;
+    }
+    diff_zero_slots(tm, a, T);
+    const bool hG = g.dG && P.nnzG > 0, hA = g.dA && P.nnzA > 0;
+    const int rG = L.Lx, rA = L.Lx + P.nnzG;
+    if (hG)
+        tan_stage(tm, a, t, tile, g.dG, P.nnzG, rG);
+    if (hA)
+        tan_stage(tm, a, t, tile, g.dA, P.nnzA, rA);
+    vd red[2] = {vset(0.0), vset(0.0)}; // max |rhs1| (set below), "not interior"
+    diff_scalings(tm, a, T, red);       // (its first barrier completes the rows above)
+    const vd zero = vset(0.0);
+    vd mx[1] = {vset(0.0)};
+    const auto rhs = [&](int q, vd r) {
+        r = r / adj_eq(a, T, q);
+        ROWD(T, L.rhs1 + q) = r;
+        mx[0] = vmax(mx[0], vabs(r));
+    };
+    for (int j = tm.wk; j < n; j += tm.nwk)
+    {
+        vd acc;
+        VFOR acc.v[c_] = -(g.dc ? g.dc[gi[c_] * n + j] : 0.0);
+        if (P.nnzA > 0) // (a problem without A may come without its column pointers)
+            for (int k = EI_LDG(P.Ap + j), k1 = EI_LDG(P.Ap + j + 1); k < k1; k++)
+                acc = vfnma(acc, hA ? vd(ROWD(T, rA + k)) : zero, ROWD(T, L.w + n + EI_LDG(P.Ai + k)));
+        if (P.nnzG > 0)
+            for (int k = EI_LDG(P.Gp + j), k1 = EI_LDG(P.Gp + j + 1); k < k1; k++)
+                acc = vfnma(acc, hG ? vd(ROWD(T, rG + k)) : zero, ROWD(T, L.w + zb + EI_LDG(P.zk + EI_LDG(P.Gi + k))));
+        rhs(j, acc);
+    }
+    for (int i = tm.wk; i < P.p; i += tm.nwk)
+    {
+        vd acc;
+        VFOR acc.v[c_] = g.db ? g.db[gi[c_] * P.p + i] : 0.0;
+        if (P.nnzA > 0)
+            for (int q = EI_LDG(P.Arp + i), q1 = EI_LDG(P.Arp + i + 1); q < q1; q++)
+                acc = vfnma(acc, hA ? vd(ROWD(T, rA + EI_LDG(P.Arv + q))) : zero, ROWD(T, L.w + EI_LDG(g.Arj + q)));
+        rhs(n + i, acc);
+    }
+    for (int i = tm.wk; i < P.m; i += tm.nwk)
+    {
+        vd acc;
+        VFOR acc.v[c_] = g.dh ? g.dh[gi[c_] * P.m + i] : 0.0;
+        if (P.nnzG > 0)
+            for (int q = EI_LDG(P.Grp + i), q1 = EI_LDG(P.Grp + i + 1); q < q1; q++)
+                acc = vfnma(acc, hG ? vd(ROWD(T, rG + EI_LDG(P.Grv + q))) : zero, ROWD(T, L.w + EI_LDG(g.Grj + q)));
+        rhs(zb + EI_LDG(P.zk + i), acc);
+    }
+    team_max<1>(tm, mx);
+    red[0] = mx[0];
+    diff_status(tm, a, t, g.exit, valid, gi, red);
+}
+
+// After the factorisation and solveKKT (rhs1 -> sol1): [dx; dy; dz] = D^-1 sol1 (rows sol2), written with
+// ds = -W^2 dz in the original scaling.  ds comes from the equilibrated solve's dz_e = sol1_z and the scaling rows of
+// the load step: ds_e = -W_e^2 dz_e (LP rows: lpv dz_e; a cone: -eta^2 (2 wb (wb' dz_e) - J dz_e), wb = (a, q)), and
+// ds = G_equil ds_e (one G_equil per cone, so W^2 = G_equil^2 W_e^2).  Lanes not differentiated get zeros.
+EI_DEV void tile_tangent_store(const Team &tm, const KArgs &a, const TanArgs &g, int tile)
+{
+    const TileMem t = tile_mem(tm, a, tile);
+    const DevPattern &P = a.P;
+    const Layout &L = a.L;
+    double *T = t.T;
+    const int n = P.n, zb = P.n + P.p;
+    vb diff;
+    int code[VEC];
+    diff_unscale(tm, a, t, L.sol2, code, diff);
+    if (g.dx)
+        for (int j = tm.wk; j < n; j += tm.nwk)
+            diff_put(t, diff, g.dx, n, j, ROWD(T, L.sol2 + j));
+    if (g.dy)
+        for (int i = tm.wk; i < P.p; i += tm.nwk)
+            diff_put(t, diff, g.dy, P.p, i, ROWD(T, L.sol2 + n + i));
+    if (g.dz)
+        for (int i = tm.wk; i < P.m; i += tm.nwk)
+            diff_put(t, diff, g.dz, P.m, i, ROWD(T, L.sol2 + zb + EI_LDG(P.zk + i)));
+    if (g.ds)
+    {
+        for (int i = tm.wk; i < P.l; i += tm.nwk)
+        {
+            const int e = EI_LDG(P.zk + i);
+            const vd dse = vd(ROWD(T, L.lpv + e)) * vd(ROWD(T, L.sol1 + zb + e));
+            diff_put(t, diff, g.ds, P.m, i, dse * adj_eq(a, T, zb + e));
+        }
+        for (int c = tm.wk; c < P.nc; c += tm.nwk)
+        {
+            const int d = EI_LDG(P.cone_dim + c), ks = EI_LDG(P.cone_k + c), qo = EI_LDG(P.cone_q + c);
+            const int cp = L.cpar + c * CP_COUNT, i0 = ks - 2 * c; // compact index of the cone's first row
+            const vd eta2 = ROWD(T, cp + CP_ETA2), av = ROWD(T, cp + CP_A), eq = adj_eq(a, T, zb + ks);
+            const vd dz0 = ROWD(T, L.sol1 + zb + ks);
+            vd wdz = av * dz0;
+            for (int k = 1; k < d; k++)
+                wdz = vfma(vd(ROWD(T, L.cq + qo + k - 1)), vd(ROWD(T, L.sol1 + zb + ks + k)), wdz);
+            diff_put(t, diff, g.ds, P.m, i0, (-eta2 * (2.0 * av * wdz - dz0)) * eq);
+            for (int k = 1; k < d; k++)
+            {
+                const vd qk = ROWD(T, L.cq + qo + k - 1), dzk = ROWD(T, L.sol1 + zb + ks + k);
+                diff_put(t, diff, g.ds, P.m, i0 + k, (-eta2 * (2.0 * qk * wdz + dzk)) * eq);
+            }
+        }
+    }
+    diff_write_status(tm, t, g.status, code);
 }
 
 } // namespace eicos

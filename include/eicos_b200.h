@@ -202,6 +202,36 @@ int eicos_batch_adjoint_device(eicos_batch *bt, int batch, const double *d_Gs, c
                                const int *d_exitflag, const double *d_gx, const double *d_gy, const double *d_gz,
                                double *d_dc, double *d_dh, double *d_db, double *d_dG, double *d_dA, int *d_status);
 
+/* ---- derivatives of the solution map along a direction (the forward-mode tangent of a batched solve)
+ * The same linearisation and the same K0 as eicos_batch_adjoint.  For a direction v = (dc, dh, db, dG, dA) in the
+ * problem data (dG, dA: values on the pattern, CSC order) one solve per instance gives
+ *     K0 [dx; dy; dz] = [-dc - dA'y - dG'z;  db - dA x;  dh - dG x],    ds = -W^2 dz,
+ * so that G dx + ds = dh - dG x.  For a loss gradient g and the adjoint's J'g, <g, J v> = <J'g, v> up to the solve's
+ * accuracy.  One call answers one direction for every instance; the reverse mode needs one call per output.
+ *
+ * Arguments (instance-major, original scaling, z-shaped arrays in compact z order):
+ *   x [batch x n], y [batch x p], z, s [batch x m], exitflag [batch]: the forward's results (required);
+ *   dc [batch x n], dh [batch x m], db [batch x p], dG [batch x nnzG], dA [batch x nnzA]: the direction, NULL = zero
+ *   (a NULL component gives the bits of a zero one and is never read); dG / dA are allowed on both kinds of handle;
+ *   dx [batch x n], dy [batch x p], dz, ds [batch x m], status [batch]: outputs, any may be NULL;
+ *   Gs, As: the forward's per-instance matrices, as in eicos_batch_adjoint (instance-matrices handles only).
+ * The handle's current matrices and settings (nitref, linsysacc, irerrfact) apply.  Per-instance status as in
+ * eicos_batch_adjoint: 0 differentiated, 1 not optimal, 2 not interior, 3 not finite; instances with status != 0
+ * get exact zeros in every output.  Each instance's results depend on its own data only, whatever the batch, the
+ * handle's capacity or its workers.  Returns EICOS_ERR_INVALID for batch <= 0, a missing required buffer or Gs / As
+ * given to a shared-matrices handle. */
+int eicos_batch_tangent(eicos_batch *bt, int batch, const double *Gs, const double *As,
+                        const double *x, const double *y, const double *z, const double *s, const int *exitflag,
+                        const double *dc, const double *dh, const double *db, const double *dG, const double *dA,
+                        double *dx, double *dy, double *dz, double *ds, int *status);
+/* The same with DEVICE buffers (results stay in HBM).  Runs on the engine's stream (eicos_batch_stream) and returns
+ * after it has drained. */
+int eicos_batch_tangent_device(eicos_batch *bt, int batch, const double *d_Gs, const double *d_As,
+                               const double *d_x, const double *d_y, const double *d_z, const double *d_s,
+                               const int *d_exitflag, const double *d_dc, const double *d_dh, const double *d_db,
+                               const double *d_dG, const double *d_dA,
+                               double *d_dx, double *d_dy, double *d_dz, double *d_ds, int *d_status);
+
 typedef struct eicos_batch_stats
 {
     int chunks, ipm_iterations;
